@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py -- items/s of HiD-VAE's residual-quantisation hot path on B200, through the reference-shaped module API.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference] [--no-sweep]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl native|reference] [--no-sweep] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 Workload (BASELINE.json configs[4], "c5": bulk semantic-ID assignment, one GPU's share of the catalogue): a chunk of
@@ -197,6 +197,24 @@ def bind_host_memory_near(local_rank):
     return info
 
 
+DUMP_LIMIT_BYTES = 64 * 10 ** 6
+DUMP_SAMPLE_ROWS = 1 << 21
+
+
+def dump_outputs(out_dir, ids):
+    """--dump-outputs: the id table the last timed step returned, as out_dir/sem_ids.npy in float32 (ids are < 2^24, so
+    exact), for comparing two builds output for output.  A table above DUMP_LIMIT_BYTES (the gathered table of a multi-GPU
+    run) is cut to a fixed seeded sample of DUMP_SAMPLE_ROWS rows, whose indices go to sem_ids_rows.npy (float64)."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    ids = ids.cpu()
+    if ids.numel() * 4 > DUMP_LIMIT_BYTES:
+        rows = torch.randperm(ids.shape[0], generator=torch.Generator().manual_seed(0))[:DUMP_SAMPLE_ROWS].sort().values
+        np.save(os.path.join(out_dir, "sem_ids_rows.npy"), rows.numpy().astype(np.float64))
+        ids = ids[rows]
+    np.save(os.path.join(out_dir, "sem_ids.npy"), ids.numpy().astype(np.float32))
+
+
 def time_steps(fn, steps, warmup, flush=None):
     """W warm-ups, then K steps each bracketed by CUDA events on the current stream (optionally an L2 flush between
     steps); returns the per-step milliseconds."""
@@ -283,6 +301,7 @@ def run_native(args):
     total_ms = float(tm.item())
     value = world * n * args.steps / (total_ms * 1e-3)
     t_mark1 = time.time()
+    last_ids = tok.cached_ids.cpu() if args.dump_outputs and rank == 0 else None   # what the last timed step returned
 
     # ---- e2e: the same call on PINNED HOST items: chunk H2D + kernels + D2H of the id table inside the timed region ----
     n_e = min(E2E_ITEMS, n)
@@ -412,6 +431,8 @@ def run_native(args):
             line["sweep"] = sweep
         if train_dp is not None:
             line["train_dp"] = train_dp
+        if last_ids is not None:
+            dump_outputs(args.dump_outputs, last_ids)
         OUT.emit(json.dumps(line))
     if world > 1:
         torch.cuda.synchronize()
@@ -744,13 +765,15 @@ def run_reference(args):
     torch.set_num_threads(cores)
     enc_w, _cb_w, cbs = _cpu_model()
     xs = synth_items(REF_SAMPLE_ITEMS, seed=1000, device="cpu")
-    steps, warmup = max(1, min(args.steps, 100)), min(args.warmup, 5)
+    steps, warmup = args.steps, min(args.warmup, 5)
     for _ in range(warmup):
         OH.precompute_corpus_ids(xs, enc_w, cbs, True)
     t0 = time.perf_counter()
     for _ in range(steps):
-        OH.precompute_corpus_ids(xs, enc_w, cbs, True)
+        ids = OH.precompute_corpus_ids(xs, enc_w, cbs, True)
     dt = time.perf_counter() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, ids)
     value = REF_SAMPLE_ITEMS * steps / dt
     sample = (f"{steps} steps x {REF_SAMPLE_ITEMS} items of the same synthetic catalogue, batches of 512 like the reference "
               f"(oracle/hrqvae.py, torch {torch.__version__} CPU, {cores} threads)")
@@ -797,7 +820,10 @@ def main():
     ap.add_argument("--impl", default="native", choices=["native", "reference"])
     ap.add_argument("--no-sweep", action="store_true")
     ap.add_argument("--chunk-items", type=int, default=CHUNK_ITEMS, help="items per launch inside precompute_corpus_ids (tuning runs)")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the id table of the last timed step to DIR/sem_ids.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     globals()["CHUNK_ITEMS"] = WORKLOAD["chunk_items"] = args.chunk_items
     args.warmup = max(args.warmup, 3) if args.impl == "native" else args.warmup
     with QuietStdout() as OUT:

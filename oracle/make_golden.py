@@ -218,7 +218,23 @@ def make_hrqvae_forward_cases(ref):
                 q = model.get_semantic_ids(model.encode(x))
                 out[f"{tag}/eval_sem_ids"] = _np(q.sem_ids)
                 out[f"{tag}/eval_tag_predictions"] = _np(model.predict_tags(x)["predictions"])
+    tags = [f"{m}_train{int(tr)}" for m in ("ste", "rot") for tr in (True, False)]
+    _store_shared_once(out, tags, lambda name: name.startswith("state/") or name in ("x", "tags_emb", "tags_indices"))
     np.savez_compressed(os.path.join(OUT, "hrqvae_forward.npz"), **out)
+
+
+def _store_shared_once(out, tags, eligible):
+    """Every case starts from the same seed, so weights and inputs repeat across cases: an eligible `<tag>/<name>`
+    that is identical under every tag is stored once as `<name>` (keeps the fixture small).  What differs, such as
+    the BatchNorm statistics a training-mode forward updates, stays under its tag."""
+    for name in [k[len(tags[0]) + 1:] for k in out if k.startswith(tags[0] + "/")]:
+        if not eligible(name):
+            continue
+        vals = [out[f"{tag}/{name}"] for tag in tags]
+        if all(v.dtype == vals[0].dtype and np.array_equal(v, vals[0]) for v in vals[1:]):
+            out[name] = vals[0]
+            for tag in tags:
+                del out[f"{tag}/{name}"]
 
 
 def make_tokenizer_cases(ref):

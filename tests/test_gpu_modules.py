@@ -88,8 +88,10 @@ def _load_reference_model(mods, g, tag, mname):
     for m in model.modules():               # same as the recording run: no dropout noise in the training-mode case
         if isinstance(m, torch.nn.Dropout):
             m.p = 0.0
+    # weights shared by every case are stored once under state/; <tag>/state/ holds what the case's own forward changed
+    state = {k[len("state/"):]: t(g[k]) for k in g.files if k.startswith("state/")}
     prefix = f"{tag}/state/"
-    state = {k[len(prefix):]: t(g[k]) for k in g.files if k.startswith(prefix)}
+    state.update({k[len(prefix):]: t(g[k]) for k in g.files if k.startswith(prefix)})
     missing, unexpected = model.load_state_dict(state, strict=True), None   # the reference's keys, unchanged
     return model.cuda()
 
@@ -101,8 +103,8 @@ def test_hrqvae_forward_with_reference_weights(mods, golden_dir, mname, training
     tag = f"{mname}_train{training}"
     model = _load_reference_model(mods, g, tag, mname)
     model.train(bool(training))
-    batch = mods.TaggedSeqBatch(None, None, None, t(g[f"{tag}/x"]).cuda(), None, None, t(g[f"{tag}/tags_emb"]).cuda(),
-                                t(g[f"{tag}/tags_indices"]).cuda())
+    batch = mods.TaggedSeqBatch(None, None, None, t(g["x"]).cuda(), None, None, t(g["tags_emb"]).cuda(),
+                                t(g["tags_indices"]).cuda())
     out = model(batch, gumbel_t=0.2)
     tol = dict(rtol=2e-4, atol=2e-5)  # encoder/decoder GEMMs run on cuBLAS (TF32 off) vs the reference's CPU sgemm
     for name in ("reconstruction_loss", "rqvae_loss", "embs_norm"):
@@ -211,7 +213,7 @@ def test_tokenizer_precompute_corpus_ids(mods, golden_dir):
     g = npz(golden_dir, "hrqvae_forward.npz")
     tag = "rot_train0"
     model = _load_reference_model(mods, g, tag, "rot")
-    x = t(g[f"{tag}/x"]).cuda()
+    x = t(g["x"]).cuda()
     for kw, width in ((dict(use_concatenated_ids=True), 6), (dict(use_interleaved_ids=True), 6), (dict(), 3)):
         tok = mods.HSemanticIdTokenizer(input_dim=64, output_dim=32, hidden_dims=[48, 40], codebook_size=64, n_layers=3,
                                         n_cat_feats=0, hrqvae_codebook_normalize=True, tag_class_counts=[5, 7, 9],
