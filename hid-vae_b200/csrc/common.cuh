@@ -97,13 +97,36 @@ __device__ __forceinline__ float fast_inv_norm_floor(float v, float floor) {
   return fast_rcp(fmaxf(s, floor));
 }
 
+// Scalars of one rotation-trick level (modules/quantize.py:34-45) from the three row sums rr = r.r, ee = e.e, re = r.e.
+// o = r - 2 (r.w) w + 2 (r.u) q with u = r ir, q = e ie, w = (u + q) is collapses to  o = cr r + ce e:
+//   r.u = rr ir,  r.q = re ie,  |u + q|^2 = rr ir^2 + ee ie^2 + 2 re ir ie,
+//   a2 = 2 (r.u + r.q) is^2,  cr = 1 - a2 ir,  ce = (2 r.u - a2) ie.
+// Two passes over the row instead of five.  |u + q|^2 from the row sums already at hand has an absolute error of ~4e-7 on a
+// value in [0, 4], i.e. 1e-7 relative on 1/|s| away from r = -e.  The forward and the backward's recomputation of the
+// chain both call this, so they agree to the bit.
+struct RotCoeffs {
+  float ir, ie, is, cr, ce;
+};
+__device__ __forceinline__ RotCoeffs rot_coeffs(float rr, float ee, float re) {
+  RotCoeffs c;
+  c.ir = fast_inv_norm_eps(rr, 1e-8f);  // u = r / (|r| + 1e-8)
+  c.ie = fast_inv_norm_eps(ee, 1e-8f);  // q = e / (|e| + 1e-8)
+  const float ru = rr * c.ir, rq = re * c.ie;
+  const float ss = fmaf(2.0f * rq, c.ir, fmaf(ru, c.ir, ee * c.ie * c.ie));
+  c.is = fast_inv_norm_floor(ss, 1e-6f);  // w = (u + q) / max(|u + q|, 1e-6)
+  const float a2 = 2.0f * (ru + rq) * c.is * c.is;
+  c.cr = 1.0f - a2 * c.ir;
+  c.ce = (2.0f * ru - a2) * c.ie;
+  return c;
+}
+
 // ---------------------------------------------------------------------------------------------------------
 // Per-row "tail" of one quantiser level: everything after the argmin.  One thread owns one row in registers.
 //   r      in : residual entering the level (r_l)            out: r_{l+1} = r_l - o_l
 //   e         : the chosen code row C_l[id] (fp32)
 //   returns the level loss a + beta*a with a = |r - e|^2      (modules/loss.py:41-44)
 //   o (emb_out) is written to `o_out` when non-null.
-// ROT implements modules/quantize.py:34-45,134-140:  o = r - 2 (r.w) w + 2 (r.u) q  (collapsed to two row passes, below)
+// ROT implements modules/quantize.py:34-45,134-140:  o = r - 2 (r.w) w + 2 (r.u) q  (collapsed to two row passes, rot_coeffs)
 // ---------------------------------------------------------------------------------------------------------
 template <int D, bool ROT>
 __device__ __forceinline__ float rq_level_tail_o(float (&r)[D], const float (&e)[D], float beta, float (&o)[D]) {
@@ -118,27 +141,15 @@ __device__ __forceinline__ float rq_level_tail_o(float (&r)[D], const float (&e)
 #pragma unroll
     for (int i = 0; i < D; ++i) o[i] = e[i];
   } else {
-    // o = r - 2 (r.w) w + 2 (r.u) q with u = r ir, q = e ie, w = (u + q) is collapses to  o = cr r + ce e  with scalars
-    // that follow from the three row sums r.r, e.e, r.e (r.e from the loss sum: |r - e|^2 = r.r + e.e - 2 r.e):
-    //   r.u = rr ir,  r.q = re ie,  |u + q|^2 = rr ir^2 + ee ie^2 + 2 re ir ie,
-    //   a2 = 2 (r.u + r.q) is^2,  cr = 1 - a2 ir,  ce = (2 r.u - a2) ie.
-    // Two passes over the row instead of five (the backward recomputes the chain with the same expressions).
     float rr = 0.f, ee = 0.f;
 #pragma unroll
     for (int i = 0; i < D; ++i) {
       rr = fmaf(r[i], r[i], rr);
       ee = fmaf(e[i], e[i], ee);
     }
-    const float re = 0.5f * ((rr + ee) - a);
-    const float inv_r = fast_inv_norm_eps(rr, 1e-8f);  // u = r / (|r| + 1e-8)
-    const float inv_e = fast_inv_norm_eps(ee, 1e-8f);  // q = e / (|e| + 1e-8)
-    const float ru = rr * inv_r, rq = re * inv_e;
-    const float ss = fmaf(2.0f * rq, inv_r, fmaf(ru, inv_r, ee * inv_e * inv_e));
-    const float inv_s = fast_inv_norm_floor(ss, 1e-6f);  // w = (u + q) / max(|u + q|, 1e-6)
-    const float a2 = 2.0f * (ru + rq) * inv_s * inv_s;
-    const float cr = 1.0f - a2 * inv_r, ce = (2.0f * ru - a2) * inv_e;
+    const RotCoeffs c = rot_coeffs(rr, ee, 0.5f * ((rr + ee) - a));  // r.e from the loss sum: |r - e|^2 = r.r + e.e - 2 r.e
 #pragma unroll
-    for (int i = 0; i < D; ++i) o[i] = fmaf(cr, r[i], ce * e[i]);
+    for (int i = 0; i < D; ++i) o[i] = fmaf(c.cr, r[i], c.ce * e[i]);
   }
 #pragma unroll
   for (int i = 0; i < D; ++i) r[i] = r[i] - o[i];

@@ -229,26 +229,6 @@ __device__ __forceinline__ void tmem_ld_32x32(uint32_t taddr, uint32_t (&v)[32])
       : "memory");
 }
 
-// 32 lanes x 16 consecutive fp32 columns
-__device__ __forceinline__ void tmem_ld_32x16(uint32_t taddr, uint32_t (&v)[16]) {
-  asm volatile(
-      "tcgen05.ld.sync.aligned.32x32b.x16.b32 "
-      "{%0, %1, %2, %3, %4, %5, %6, %7, %8, %9, %10, %11, %12, %13, %14, %15}, [%16];"
-      : "=r"(v[0]), "=r"(v[1]), "=r"(v[2]), "=r"(v[3]), "=r"(v[4]), "=r"(v[5]), "=r"(v[6]), "=r"(v[7]), "=r"(v[8]),
-        "=r"(v[9]), "=r"(v[10]), "=r"(v[11]), "=r"(v[12]), "=r"(v[13]), "=r"(v[14]), "=r"(v[15])
-      : "r"(taddr)
-      : "memory");
-}
-__device__ __forceinline__ void tmem_wait_ld(uint32_t (&v)[16], uint32_t (&w)[16]) {
-  asm volatile("tcgen05.wait::ld.sync.aligned;"
-               : "+r"(v[0]), "+r"(v[1]), "+r"(v[2]), "+r"(v[3]), "+r"(v[4]), "+r"(v[5]), "+r"(v[6]), "+r"(v[7]), "+r"(v[8]),
-                 "+r"(v[9]), "+r"(v[10]), "+r"(v[11]), "+r"(v[12]), "+r"(v[13]), "+r"(v[14]), "+r"(v[15]), "+r"(w[0]),
-                 "+r"(w[1]), "+r"(w[2]), "+r"(w[3]), "+r"(w[4]), "+r"(w[5]), "+r"(w[6]), "+r"(w[7]), "+r"(w[8]),
-                 "+r"(w[9]), "+r"(w[10]), "+r"(w[11]), "+r"(w[12]), "+r"(w[13]), "+r"(w[14]), "+r"(w[15])
-               :
-               : "memory");
-}
-
 __device__ __forceinline__ void tmem_wait_ld16(uint32_t (&v)[16]) {
   asm volatile("tcgen05.wait::ld.sync.aligned;"
                : "+r"(v[0]), "+r"(v[1]), "+r"(v[2]), "+r"(v[3]), "+r"(v[4]), "+r"(v[5]), "+r"(v[6]), "+r"(v[7]), "+r"(v[8]),

@@ -1,15 +1,15 @@
 // Fused backward of the L-level residual quantiser (STE / rotation trick / eval) -- HBM-bound, no GEMM.
 //
-// One pass over the rows.  A row is spread over D/4 lanes (one float4 each) so every global access of a warp
+// One pass over the rows.  A row is spread over D/W lanes (W = 4 or 8 floats each, Frag) so every global access of a warp
 // is a run of contiguous 16-byte pieces; dot products are reduced with xor-shuffles inside the lane group.
-// The forward chain r_l, e_l is recomputed from x, ids and the codebooks (nothing was saved by the forward),
-// then the recursion of SURVEY.md section 8a runs from the last level to the first:
+// The forward chain r_l, e_l is recomputed from x, ids and the codebooks (nothing was saved by the forward; level_forward),
+// then the recursion of SURVEY.md section 8a runs from the last level to the first (level_backward):
 //     h   = g_emb_l - G                      (G = dLoss/d r_{l+1})
 //     Jh  = h                                (STE)      | h - 2 (h.w) w + 2 (h.q) u   (rotation trick)
 //     G   = G + Jh + 2 beta (r_l - e_l) g_loss          | eval: G = G + 2 beta (r_l - e_l) g_loss
 //     gC_l[id_l] += 2 (e_l - r_l) g_loss                | eval: += h + 2 (e_l - r_l) g_loss
 // The codebook gradient is a scatter-add by id (the embedding_dense_backward of modules/quantize.py:97-98): one
-// red.global.add.v4.f32 per lane, spread over zeroed replicas of [L, K, D] for large N (folded by a second tiny kernel).
+// red.global.add.v4.f32 per 16-byte piece, spread over zeroed replicas of [L, K, D] for large N (folded by a second tiny kernel).
 #include <stdlib.h>
 
 #include <type_traits>
@@ -22,9 +22,7 @@ namespace {
 
 constexpr int kMaxLevels = 8;
 constexpr int kBwdThreads = 256;
-#ifndef HV_BWD_MINB
-#define HV_BWD_MINB 3  // CTAs per SM the exact-level instantiations are compiled for (register cap 80)
-#endif
+constexpr int kBwdMinBlocks = 3;  // CTAs per SM the exact-level row-kernel instantiations are compiled for (register cap 80)
 
 struct RqBwdArgs {
   const float* x;
@@ -56,20 +54,130 @@ __device__ __forceinline__ float group_sum(float v) {
   return v;
 }
 
-// one 16-byte reduction per lane instead of four scalar atomics (sm_90+: red.global.add.v4.f32)
-__device__ __forceinline__ void red_add_v4(float* addr, const float4& v) {
-  asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(addr), "f"(v.x), "f"(v.y), "f"(v.z), "f"(v.w) : "memory");
+// A lane's W floats of a row.  W = 4: one 16-byte piece, dims [4 sub, 4 sub + 4).  W = 8: two pieces HALF A ROW apart (those
+// dims and D/2 + the same), so that the lanes of a row cover whole 32-byte sectors with each instruction.  The helpers below
+// take the row's first element and the lane's index in the row's lane group.
+template <int W>
+struct Frag {
+  static_assert(W == 4 || W == 8, "four or eight floats per lane");
+  float v[W];
+};
+
+// piece j of the lane: float4 number sub + j D/8 of the row
+template <int D, int W>
+__device__ __forceinline__ Frag<W> ldg_frag(const float* row, int sub) {
+  Frag<W> f;
+  const float4 t = __ldg(reinterpret_cast<const float4*>(row) + sub);
+  f.v[0] = t.x, f.v[1] = t.y, f.v[2] = t.z, f.v[3] = t.w;
+  if constexpr (W == 8) {
+    const float4 u = __ldg(reinterpret_cast<const float4*>(row) + sub + D / 8);
+    f.v[4] = u.x, f.v[5] = u.y, f.v[6] = u.z, f.v[7] = u.w;
+  }
+  return f;
+}
+template <int D, int W>
+__device__ __forceinline__ Frag<W> lds_frag(const float* row, int sub) {
+  Frag<W> f;
+  const float4 t = reinterpret_cast<const float4*>(row)[sub];
+  f.v[0] = t.x, f.v[1] = t.y, f.v[2] = t.z, f.v[3] = t.w;
+  if constexpr (W == 8) {
+    const float4 u = reinterpret_cast<const float4*>(row)[sub + D / 8];
+    f.v[4] = u.x, f.v[5] = u.y, f.v[6] = u.z, f.v[7] = u.w;
+  }
+  return f;
+}
+template <int D, int W>
+__device__ __forceinline__ void store_frag(float* row, int sub, const Frag<W>& f) {
+  reinterpret_cast<float4*>(row)[sub] = make_float4(f.v[0], f.v[1], f.v[2], f.v[3]);
+  if constexpr (W == 8) reinterpret_cast<float4*>(row)[sub + D / 8] = make_float4(f.v[4], f.v[5], f.v[6], f.v[7]);
+}
+// one 16-byte reduction per piece instead of four scalar atomics (sm_90+: red.global.add.v4.f32)
+__device__ __forceinline__ void red_add_v4(float* addr, float x, float y, float z, float w) {
+  asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(addr), "f"(x), "f"(y), "f"(z), "f"(w) : "memory");
+}
+template <int D, int W>
+__device__ __forceinline__ void red_add_frag(float* base, int64_t row_off, int sub, const Frag<W>& f) {  // row = base + row_off
+  float* p = base + (row_off + sub * 4);
+  red_add_v4(p, f.v[0], f.v[1], f.v[2], f.v[3]);
+  if constexpr (W == 8) red_add_v4(p + D / 2, f.v[4], f.v[5], f.v[6], f.v[7]);
+}
+// the lane's part of a dot product: one fmaf chain at W = 4, two accumulators at W = 8
+template <int W>
+__device__ __forceinline__ float dot(const Frag<W>& a, const Frag<W>& b) {
+  if constexpr (W == 4) {
+    return fmaf(a.v[0], b.v[0], fmaf(a.v[1], b.v[1], fmaf(a.v[2], b.v[2], a.v[3] * b.v[3])));
+  } else {
+    float s0 = a.v[0] * b.v[0], s1 = a.v[1] * b.v[1];
+#pragma unroll
+    for (int i = 2; i < W; i += 2) s0 = fmaf(a.v[i], b.v[i], s0), s1 = fmaf(a.v[i + 1], b.v[i + 1], s1);
+    return s0 + s1;
+  }
 }
 
-__device__ __forceinline__ float dot4(const float4& a, const float4& b) {
-  return fmaf(a.x, b.x, fmaf(a.y, b.y, fmaf(a.z, b.z, a.w * b.w)));
+// One level of the recomputed forward chain: r_l -> r_{l+1} = r_l - o_l with o = e (STE, eval) or o = cr r + ce e (rotation
+// trick, modules/quantize.py:34-45), whose scalars are kept in `c` for the backward.  r.r, e.e and r.e are the only row sums
+// (3 shuffle reductions instead of 5).
+template <int LPR, int W, bool ROT>
+__device__ __forceinline__ void level_forward(Frag<W>& r, const Frag<W>& e, RotCoeffs& c) {
+  Frag<W> o = e;
+  if constexpr (ROT) {
+    const float rr = group_sum<LPR>(dot(r, r));
+    const float ee = group_sum<LPR>(dot(e, e));
+    const float re = group_sum<LPR>(dot(r, e));
+    c = rot_coeffs(rr, ee, re);
+#pragma unroll
+    for (int i = 0; i < W; ++i) o.v[i] = fmaf(c.cr, r.v[i], c.ce * e.v[i]);
+  }
+#pragma unroll
+  for (int i = 0; i < W; ++i) r.v[i] -= o.v[i];
 }
 
+// One step of the recursion at level l (rl = r_l, el = e_l, ge = g_emb_l, gl = the level's loss gradient): G becomes
+// dLoss/d r_l; returns the lane's piece of the gradient of the code row e_l.
+template <int LPR, int W, bool ROT, bool TRAIN>
+__device__ __forceinline__ Frag<W> level_backward(Frag<W>& G, const Frag<W>& ge, const Frag<W>& rl, const Frag<W>& el,
+                                                  const RotCoeffs& c, float gl, float beta) {
+  Frag<W> h, diff, ge_code;
+#pragma unroll
+  for (int i = 0; i < W; ++i) h.v[i] = ge.v[i] - G.v[i];
+#pragma unroll
+  for (int i = 0; i < W; ++i) diff.v[i] = rl.v[i] - el.v[i];
+  const float c2 = 2.0f * gl;
+#pragma unroll
+  for (int i = 0; i < W; ++i) ge_code.v[i] = -c2 * diff.v[i];
+  const float cb2 = beta * c2;
+  if constexpr (TRAIN) {
+    if constexpr (ROT) {  // Jh with u = r ir, q = e ie, w = (u + q) is
+      Frag<W> u, q, w;
+#pragma unroll
+      for (int i = 0; i < W; ++i) u.v[i] = rl.v[i] * c.ir;
+#pragma unroll
+      for (int i = 0; i < W; ++i) q.v[i] = el.v[i] * c.ie;
+#pragma unroll
+      for (int i = 0; i < W; ++i) w.v[i] = (u.v[i] + q.v[i]) * c.is;
+      const float hw2 = 2.0f * group_sum<LPR>(dot(h, w));
+      const float hq2 = 2.0f * group_sum<LPR>(dot(h, q));
+#pragma unroll
+      for (int i = 0; i < W; ++i) h.v[i] = h.v[i] - hw2 * w.v[i] + hq2 * u.v[i];
+    }
+#pragma unroll
+    for (int i = 0; i < W; ++i) G.v[i] += h.v[i] + cb2 * diff.v[i];
+  } else {
+#pragma unroll
+    for (int i = 0; i < W; ++i) G.v[i] += cb2 * diff.v[i];
+#pragma unroll
+    for (int i = 0; i < W; ++i) ge_code.v[i] += h.v[i];
+  }
+  return ge_code;
+}
+
+// Row kernel: four floats per lane, code rows gathered from global memory.
 // NL > 0: exactly NL levels, known at compile time (no per-level branches, register arrays of that size; 1..4 cover
 // every shipped config and keep the kernel at 3+ CTAs per SM); NL == 0: runtime level count up to kMaxLevels.
 // ROT / TRAIN: rotation-trick Jacobian / training semantics (eval: emb_out = e for every mode, quantize.py:146-147).
 template <int D, bool ROT, bool TRAIN, int NL>
-__global__ void __launch_bounds__(kBwdThreads, NL > 0 ? HV_BWD_MINB : 1) rq_bwd_kernel(RqBwdArgs a) {
+__global__ void __launch_bounds__(kBwdThreads, NL > 0 ? kBwdMinBlocks : 1) rq_bwd_kernel(RqBwdArgs a) {
+  static_assert(TRAIN || !ROT, "eval has no rotation");
   constexpr int LMAX = NL > 0 ? NL : kMaxLevels;
   constexpr int LPR = D / 4;  // lanes per row
   constexpr int ROWS_PER_WARP = 32 / LPR;
@@ -80,7 +188,6 @@ __global__ void __launch_bounds__(kBwdThreads, NL > 0 ? HV_BWD_MINB : 1) rq_bwd_
   const int warp_global = ptx::uniform((blockIdx.x * kBwdThreads + threadIdx.x) >> 5);  // (see ptx::warp_index)
   const int n_warps = (gridDim.x * kBwdThreads) >> 5;
   const int64_t n_groups = (a.n + ROWS_PER_WARP - 1) / ROWS_PER_WARP;
-  constexpr bool rot = ROT && TRAIN;
   float* gc_base = a.n_replicas > 0 ? a.replicas + static_cast<int64_t>(blockIdx.x % a.n_replicas) * lkd : a.g_codebooks;
 
   for (int64_t g = warp_global; g < n_groups; g += n_warps) {
@@ -88,133 +195,84 @@ __global__ void __launch_bounds__(kBwdThreads, NL > 0 ? HV_BWD_MINB : 1) rq_bwd_
     const bool valid = row < a.n;
     const int64_t rrow = valid ? row : 0;  // keep every lane in the shuffles; mask the stores
 
-    float4 R[LMAX], E[LMAX];
-    float inv_r[LMAX], inv_e[LMAX], inv_s[LMAX];
+    Frag<4> R[LMAX], E[LMAX];
+    RotCoeffs rc[LMAX];
     int id[LMAX];
-    float4 r = __ldg(reinterpret_cast<const float4*>(a.x + rrow * D) + sub);
+    Frag<4> r = ldg_frag<D, 4>(a.x + rrow * D, sub);
 #pragma unroll
     for (int l = 0; l < LMAX; ++l) {
       if (NL > 0 || l < a.n_levels) {
         int64_t code = a.ids[rrow * a.ids_row_stride + l * a.ids_level_stride];
         code = code < 0 ? 0 : (code >= a.k ? a.k - 1 : code);
         id[l] = static_cast<int>(code);
-        const float4 e = __ldg(reinterpret_cast<const float4*>(a.codebooks + (static_cast<int64_t>(l) * a.k + code) * D) + sub);
+        E[l] = ldg_frag<D, 4>(a.codebooks + (static_cast<int64_t>(l) * a.k + code) * D, sub);
         R[l] = r;
-        E[l] = e;
-        float4 o = e;
-        if (rot) {
-          // modules/quantize.py:34-45 with u = r ir, q = e ie, s = u + q.  r.u = rr ir, r.s = rr ir + re ie and |s|^2 all
-          // follow from the three row sums r.r, e.e, r.e (3 shuffle reductions instead of 5)
-          const float rr = group_sum<LPR>(dot4(r, r));
-          const float ee = group_sum<LPR>(dot4(e, e));
-          const float re = group_sum<LPR>(dot4(r, e));
-          const float ir = fast_inv_norm_eps(rr, 1e-8f);
-          const float ie = fast_inv_norm_eps(ee, 1e-8f);
-          const float ru = rr * ir;
-          const float rq = re * ie;
-          // |u + q|^2 = |u|^2 + |q|^2 + 2 u.q from the three row sums already at hand (one shuffle reduction and a vector
-          // pass less per level; absolute error ~4e-7 on a value in [0, 4], i.e. 1e-7 relative on 1/|s| away from r = -e)
-          const float ss = fmaf(2.0f * rq, ir, fmaf(ru, ir, ee * ie * ie));
-          const float rs = ru + rq;
-          const float is = fast_inv_norm_floor(ss, 1e-6f);
-          inv_r[l] = ir, inv_e[l] = ie, inv_s[l] = is;
-          // o = r - 2 (r.w) w + 2 (r.u) q  with w = (u + q) is:   o = r (1 - a ir) + e (b - a) ie,  a = 2 rs is^2, b = 2 ru
-          const float a2 = 2.0f * rs * is * is, b2 = 2.0f * ru;
-          const float cr = 1.0f - a2 * ir, ce = (b2 - a2) * ie;
-          o.x = fmaf(cr, r.x, ce * e.x);
-          o.y = fmaf(cr, r.y, ce * e.y);
-          o.z = fmaf(cr, r.z, ce * e.z);
-          o.w = fmaf(cr, r.w, ce * e.w);
-        }
-        r = make_float4(r.x - o.x, r.y - o.y, r.z - o.z, r.w - o.w);
+        level_forward<LPR, 4, ROT>(r, E[l], rc[l]);
       }
     }
 
     // every load of the row is issued before the recursion (the red.add below orders memory, so nothing can be
     // hoisted across it by the compiler): one latency exposure per row instead of one per level
     const float gl_all = a.g_loss != nullptr ? a.g_loss[rrow * a.g_loss_stride] : 0.f;
-    float4 GE[LMAX];
+    Frag<4> GE[LMAX];
     float GL[LMAX];
 #pragma unroll
     for (int l = 0; l < LMAX; ++l) {
-      GE[l] = make_float4(0.f, 0.f, 0.f, 0.f);
+      GE[l] = Frag<4>{};
       GL[l] = gl_all;
       if (NL > 0 || l < a.n_levels) {
-        if (a.g_emb != nullptr)
-          GE[l] = __ldg(reinterpret_cast<const float4*>(a.g_emb + l * a.g_emb_level_stride + rrow * a.g_emb_row_stride) + sub);
+        if (a.g_emb != nullptr) GE[l] = ldg_frag<D, 4>(a.g_emb + l * a.g_emb_level_stride + rrow * a.g_emb_row_stride, sub);
         if (a.g_level_loss != nullptr) GL[l] += a.g_level_loss[static_cast<int64_t>(l) * a.n + rrow];
       }
     }
-    float4 G = make_float4(0.f, 0.f, 0.f, 0.f);
+    Frag<4> G{};
 #pragma unroll
     for (int l = LMAX - 1; l >= 0; --l) {
       if (NL > 0 || l < a.n_levels) {
-        const float gl = GL[l];
-        const float4 ge = GE[l];
-        float4 h = make_float4(ge.x - G.x, ge.y - G.y, ge.z - G.z, ge.w - G.w);
-        const float4 rl = R[l], el = E[l];
-        const float4 diff = make_float4(rl.x - el.x, rl.y - el.y, rl.z - el.z, rl.w - el.w);
-        const float c2 = 2.0f * gl;
-        float4 ge_code = make_float4(-c2 * diff.x, -c2 * diff.y, -c2 * diff.z, -c2 * diff.w);
-        const float cb2 = a.beta * c2;
-        if (TRAIN) {
-          float4 jh = h;
-          if (rot) {
-            const float ir = inv_r[l], ie = inv_e[l], is = inv_s[l];
-            const float4 u = make_float4(rl.x * ir, rl.y * ir, rl.z * ir, rl.w * ir);
-            const float4 q = make_float4(el.x * ie, el.y * ie, el.z * ie, el.w * ie);
-            const float4 w = make_float4((u.x + q.x) * is, (u.y + q.y) * is, (u.z + q.z) * is, (u.w + q.w) * is);
-            const float hw2 = 2.0f * group_sum<LPR>(dot4(h, w));
-            const float hq2 = 2.0f * group_sum<LPR>(dot4(h, q));
-            jh.x = h.x - hw2 * w.x + hq2 * u.x;
-            jh.y = h.y - hw2 * w.y + hq2 * u.y;
-            jh.z = h.z - hw2 * w.z + hq2 * u.z;
-            jh.w = h.w - hw2 * w.w + hq2 * u.w;
-          }
-          G.x += jh.x + cb2 * diff.x, G.y += jh.y + cb2 * diff.y;
-          G.z += jh.z + cb2 * diff.z, G.w += jh.w + cb2 * diff.w;
-        } else {
-          G.x += cb2 * diff.x, G.y += cb2 * diff.y, G.z += cb2 * diff.z, G.w += cb2 * diff.w;
-          ge_code.x += h.x, ge_code.y += h.y, ge_code.z += h.z, ge_code.w += h.w;
-        }
-        if (valid) {
-          const int64_t off = (static_cast<int64_t>(l) * a.k + id[l]) * D + sub * 4;
-          red_add_v4(gc_base + off, ge_code);
-        }
+        const Frag<4> ge_code = level_backward<LPR, 4, ROT, TRAIN>(G, GE[l], R[l], E[l], rc[l], GL[l], a.beta);
+        if (valid) red_add_frag<D>(gc_base, (static_cast<int64_t>(l) * a.k + id[l]) * D, sub, ge_code);
       }
     }
-    if (valid) reinterpret_cast<float4*>(a.g_x + row * D)[sub] = G;
+    if (valid) store_frag<D>(a.g_x + row * D, sub, G);
   }
 }
 
 // ---------------------------------------------------------------------------------------------------------------------
-// Large-N variant for codebooks that fit in shared memory (L K D 4 <= 96 KB: every HiD-VAE config).  Same arithmetic, two
-// changes that remove the memory latency the kernel above exposes per row (ncu: stall_long_scoreboard 39 % of warp time):
+// Large-N kernel for codebooks that fit in shared memory (L K D 4 <= 96 KB: every HiD-VAE config).  Same arithmetic as the
+// row kernel, without the memory latency that kernel exposes per row (ncu: stall_long_scoreboard 39 % of warp time):
 //   * the fp32 codebooks are staged in shared memory once per persistent CTA: the id -> code row gather
-//     is an LDS.128 instead of a dependent round trip to L2 (and 4 L D bytes per row less L2 traffic);
+//     is an LDS.128 instead of a dependent round trip to L2 (and 4 L D bytes per row less L2 traffic), and the backward
+//     sweep reads the chosen code rows from there a second time instead of keeping them in registers;
 //   * the row's inputs (x, ids, g_emb, g_loss) are loaded ONE ITERATION AHEAD into registers, so no load of the current
 //     row is ever waited for.
+// W = 8 serves the rotation trick in training.  At W = 4 that chain is bound by issue slots (ncu: 70 % issue utilisation,
+// 554 instructions per 4 rows), and about half of them are the per-row scalars -- shuffle reductions, three reciprocal norms,
+// the rotation coefficients -- that every lane of a row repeats.  With half as many lanes per row each of those warp
+// instructions serves twice as many rows and a reduction is one shuffle shorter.
 // ---------------------------------------------------------------------------------------------------------------------
-// (one CTA of 512 threads per SM: STE training backward at 4 Mi rows 0.674 ms at 2 x 320 threads, 0.642 at 1 x 384, 0.600 at
-// 1 x 512; the eight-floats-per-lane kernel below measures 0.708 on this chain -- it pays off where the per-row scalars dominate)
-#ifndef HV_BWD2_THREADS
-#define HV_BWD2_THREADS 512
-#endif
-#ifndef HV_BWD2_CTAS
-#define HV_BWD2_CTAS 1
-#endif
-constexpr int kBwd2Threads = HV_BWD2_THREADS;
-constexpr int kBwd2SmemLimit = 96 * 1024;
+// One CTA per SM, of
+//   W = 4: 512 threads.  STE training backward at 4 Mi rows: 0.674 ms at 2 x 320 threads, 0.642 at 1 x 384, 0.600 at 1 x 512;
+//          the W = 8 kernel measures 0.708 on this chain -- it pays off where the per-row scalars dominate.
+//   W = 8: 384 threads, i.e. 168 registers per thread: nothing spills and the compiler keeps more of the chain in registers.
+//          Measured at 4 Mi rows (D = 32, L = 3): 2 x 256 threads (128 registers, 56 B of spills) 0.708 ms, 1 x 320 0.687,
+//          1 x 352 0.637, 1 x 384 0.600, 1 x 416 / 448 (152 / 144 registers) 0.84, 1 x 512 0.696, 2 x 320 1.19, 3 x 192 1.89.
+template <int W>
+constexpr int kSmemThreads = W == 8 ? 384 : 512;
+constexpr int kSmemLimit = 96 * 1024;
+// Below this many rows the row kernel runs: staging the codebooks does not pay off (a threshold of 4,096 rows measured
+// slower at 12 k and 32 k rows).
+constexpr int64_t kSmemMinRows = 65536;
 
-template <int D, bool ROT, bool TRAIN, int NL>
-__global__ void __launch_bounds__(kBwd2Threads, HV_BWD2_CTAS) rq_bwd_smem_kernel(RqBwdArgs a) {
-  constexpr int LPR = D / 4;
+template <int D, int W, bool ROT, bool TRAIN, int NL>
+__global__ void __launch_bounds__(kSmemThreads<W>, 1) rq_bwd_smem_kernel(RqBwdArgs a) {
+  static_assert(TRAIN || !ROT, "eval has no rotation");
+  constexpr int kThreads = kSmemThreads<W>;
+  constexpr int LPR = D / W;
   constexpr int ROWS_PER_WARP = 32 / LPR;
-  constexpr bool rot = ROT && TRAIN;
   extern __shared__ __align__(16) float s_cb[];  // [NL][K][D]
   {
     const int total4 = NL * a.k * (D / 4);
-    for (int i = threadIdx.x; i < total4; i += kBwd2Threads)
+    for (int i = threadIdx.x; i < total4; i += kThreads)
       reinterpret_cast<float4*>(s_cb)[i] = __ldg(reinterpret_cast<const float4*>(a.codebooks) + i);
   }
   __syncthreads();
@@ -224,27 +282,26 @@ __global__ void __launch_bounds__(kBwd2Threads, HV_BWD2_CTAS) rq_bwd_smem_kernel
   const int sub = lane % LPR;
   // (the broadcast tells the compiler that the value -- and with it the trip count of the row loop -- is warp-uniform: without it
   // every shuffle of the loop carries a WARPSYNC.COLLECTIVE / ENDCOLLECTIVE pair and register moves)
-  const int warp_global = ptx::uniform((blockIdx.x * kBwd2Threads + threadIdx.x) >> 5);
-  const int n_warps = (gridDim.x * kBwd2Threads) >> 5;
+  const int warp_global = ptx::uniform((blockIdx.x * kThreads + threadIdx.x) >> 5);
+  const int n_warps = (gridDim.x * kThreads) >> 5;
   const int64_t n_groups = (a.n + ROWS_PER_WARP - 1) / ROWS_PER_WARP;
   float* gc_base = a.n_replicas > 0 ? a.replicas + static_cast<int64_t>(blockIdx.x % a.n_replicas) * lkd : a.g_codebooks;
 
   // the next iteration's inputs
-  float4 nx, nge[NL];
+  Frag<W> nx, nge[NL];
   int nid[NL];
   float ngl;
   auto fetch = [&](int64_t g) {
     const int64_t row = g * ROWS_PER_WARP + lane / LPR;
     const int64_t rrow = row < a.n ? row : 0;  // keep every lane in the shuffles; the stores are masked
-    nx = __ldg(reinterpret_cast<const float4*>(a.x + rrow * D) + sub);
+    nx = ldg_frag<D, W>(a.x + rrow * D, sub);
     ngl = a.g_loss != nullptr ? __ldg(a.g_loss + rrow * a.g_loss_stride) : 0.f;
 #pragma unroll
     for (int l = 0; l < NL; ++l) {
       int64_t code = __ldg(a.ids + rrow * a.ids_row_stride + l * a.ids_level_stride);
       code = code < 0 ? 0 : (code >= a.k ? a.k - 1 : code);
       nid[l] = static_cast<int>(code);
-      nge[l] = a.g_emb != nullptr ? __ldg(reinterpret_cast<const float4*>(a.g_emb + l * a.g_emb_level_stride + rrow * a.g_emb_row_stride) + sub)
-                                  : make_float4(0.f, 0.f, 0.f, 0.f);
+      nge[l] = a.g_emb != nullptr ? ldg_frag<D, W>(a.g_emb + l * a.g_emb_level_stride + rrow * a.g_emb_row_stride, sub) : Frag<W>{};
     }
   };
   if (warp_global < n_groups) fetch(warp_global);
@@ -252,272 +309,38 @@ __global__ void __launch_bounds__(kBwd2Threads, HV_BWD2_CTAS) rq_bwd_smem_kernel
   for (int64_t g = warp_global; g < n_groups; g += n_warps) {
     const int64_t row = g * ROWS_PER_WARP + lane / LPR;
     const bool valid = row < a.n;
-    float4 r = nx;
+    Frag<W> r = nx;
     const float gl = ngl;
-    float4 GE[NL];
+    Frag<W> GE[NL];
     int id[NL];
 #pragma unroll
     for (int l = 0; l < NL; ++l) GE[l] = nge[l], id[l] = nid[l];
     if (g + n_warps < n_groups) fetch(g + n_warps);
+    auto code_row = [&](int l) { return s_cb + (static_cast<int64_t>(l) * a.k + id[l]) * D; };
 
-    float4 R[NL], E[NL];
-    float inv_r[NL], inv_e[NL], inv_s[NL];
+    Frag<W> R[NL];
+    RotCoeffs rc[NL];
 #pragma unroll
     for (int l = 0; l < NL; ++l) {
-      const float4 e = *reinterpret_cast<const float4*>(s_cb + (static_cast<int64_t>(l) * a.k + id[l]) * D + sub * 4);
       R[l] = r;
-      E[l] = e;
-      float4 o = e;
-      if (rot) {  // (same expressions as rq_bwd_kernel)
-        const float rr = group_sum<LPR>(dot4(r, r));
-        const float ee = group_sum<LPR>(dot4(e, e));
-        const float re = group_sum<LPR>(dot4(r, e));
-        const float ir = fast_inv_norm_eps(rr, 1e-8f);
-        const float ie = fast_inv_norm_eps(ee, 1e-8f);
-        const float ru = rr * ir;
-        const float rq = re * ie;
-        // |u + q|^2 = |u|^2 + |q|^2 + 2 u.q from the three row sums already at hand (one shuffle reduction and a vector
-        // pass less per level; absolute error ~4e-7 on a value in [0, 4], i.e. 1e-7 relative on 1/|s| away from r = -e)
-        const float ss = fmaf(2.0f * rq, ir, fmaf(ru, ir, ee * ie * ie));
-        const float rs = ru + rq;
-        const float is = fast_inv_norm_floor(ss, 1e-6f);
-        inv_r[l] = ir, inv_e[l] = ie, inv_s[l] = is;
-        const float a2 = 2.0f * rs * is * is, b2 = 2.0f * ru;
-        const float cr = 1.0f - a2 * ir, ce = (b2 - a2) * ie;
-        o.x = fmaf(cr, r.x, ce * e.x);
-        o.y = fmaf(cr, r.y, ce * e.y);
-        o.z = fmaf(cr, r.z, ce * e.z);
-        o.w = fmaf(cr, r.w, ce * e.w);
-      }
-      r = make_float4(r.x - o.x, r.y - o.y, r.z - o.z, r.w - o.w);
+      level_forward<LPR, W, ROT>(r, lds_frag<D, W>(code_row(l), sub), rc[l]);
     }
-
-    float4 G = make_float4(0.f, 0.f, 0.f, 0.f);
+    Frag<W> G{};
 #pragma unroll
     for (int l = NL - 1; l >= 0; --l) {
-      const float4 ge = GE[l];
-      float4 h = make_float4(ge.x - G.x, ge.y - G.y, ge.z - G.z, ge.w - G.w);
-      const float4 rl = R[l], el = E[l];
-      const float4 diff = make_float4(rl.x - el.x, rl.y - el.y, rl.z - el.z, rl.w - el.w);
-      const float c2 = 2.0f * gl;
-      float4 ge_code = make_float4(-c2 * diff.x, -c2 * diff.y, -c2 * diff.z, -c2 * diff.w);
-      const float cb2 = a.beta * c2;
-      if (TRAIN) {
-        float4 jh = h;
-        if (rot) {
-          const float ir = inv_r[l], ie = inv_e[l], is = inv_s[l];
-          const float4 u = make_float4(rl.x * ir, rl.y * ir, rl.z * ir, rl.w * ir);
-          const float4 q = make_float4(el.x * ie, el.y * ie, el.z * ie, el.w * ie);
-          const float4 w = make_float4((u.x + q.x) * is, (u.y + q.y) * is, (u.z + q.z) * is, (u.w + q.w) * is);
-          const float hw2 = 2.0f * group_sum<LPR>(dot4(h, w));
-          const float hq2 = 2.0f * group_sum<LPR>(dot4(h, q));
-          jh.x = h.x - hw2 * w.x + hq2 * u.x;
-          jh.y = h.y - hw2 * w.y + hq2 * u.y;
-          jh.z = h.z - hw2 * w.z + hq2 * u.z;
-          jh.w = h.w - hw2 * w.w + hq2 * u.w;
-        }
-        G.x += jh.x + cb2 * diff.x, G.y += jh.y + cb2 * diff.y;
-        G.z += jh.z + cb2 * diff.z, G.w += jh.w + cb2 * diff.w;
-      } else {
-        G.x += cb2 * diff.x, G.y += cb2 * diff.y, G.z += cb2 * diff.z, G.w += cb2 * diff.w;
-        ge_code.x += h.x, ge_code.y += h.y, ge_code.z += h.z, ge_code.w += h.w;
-      }
-      if (valid) red_add_v4(gc_base + (static_cast<int64_t>(l) * a.k + id[l]) * D + sub * 4, ge_code);
+      const Frag<W> ge_code = level_backward<LPR, W, ROT, TRAIN>(G, GE[l], R[l], lds_frag<D, W>(code_row(l), sub), rc[l], gl, a.beta);
+      if (valid) red_add_frag<D>(gc_base, (static_cast<int64_t>(l) * a.k + id[l]) * D, sub, ge_code);
     }
-    if (valid) reinterpret_cast<float4*>(a.g_x + row * D)[sub] = G;
+    if (valid) store_frag<D>(a.g_x + row * D, sub, G);
   }
 }
 
-// ---------------------------------------------------------------------------------------------------------------------
-// The same kernel with EIGHT floats of a row per lane (D / 8 lanes per row, 8 rows per warp at D = 32).  The kernel above is
-// bound by issue slots (ncu: 70 % issue utilisation, 554 instructions per 4 rows), and about half of them are the per-row
-// scalars -- shuffle reductions, three reciprocal norms, the rotation coefficients -- that every lane of a row repeats.
-// With half as many lanes per row each of those warp instructions serves twice as many rows and a reduction is one shuffle
-// shorter.  Registers: the chosen code rows are read from shared memory a second time in the backward sweep instead of
-// being kept (2 LDS.128 per level).
-// ---------------------------------------------------------------------------------------------------------------------
-// One CTA of 384 threads per SM, i.e. 168 registers per thread: nothing spills and the compiler keeps more of the chain in
-// registers.  Measured at 4 Mi rows (D = 32, L = 3): 2 x 256 threads (128 registers, 56 B of spills) 0.708 ms, 1 x 320 0.687,
-// 1 x 352 0.637, 1 x 384 0.600, 1 x 416 / 448 (152 / 144 registers) 0.84, 1 x 512 0.696, 2 x 320 1.19, 3 x 192 1.89.
-#ifndef HV_BWD8_THREADS
-#define HV_BWD8_THREADS 384
-#endif
-#ifndef HV_BWD8_CTAS
-#define HV_BWD8_CTAS 1
-#endif
-constexpr int kBwd8Threads = HV_BWD8_THREADS;
-
-struct F8 {
-  float v[8];
-};
-// a lane's eight floats of a row are two 16-byte pieces HALF A ROW apart (dims [4 sub, 4 sub + 4) and D/2 + the same): the
-// lanes of a row then cover whole 32-byte sectors with each instruction
-template <int D>
-__device__ __forceinline__ F8 ldg8(const float* p) {
-  const float4 a = __ldg(reinterpret_cast<const float4*>(p)), b = __ldg(reinterpret_cast<const float4*>(p + D / 2));
-  return F8{{a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w}};
-}
-template <int D>
-__device__ __forceinline__ F8 lds8(const float* p) {
-  const float4 a = *reinterpret_cast<const float4*>(p), b = *reinterpret_cast<const float4*>(p + D / 2);
-  return F8{{a.x, a.y, a.z, a.w, b.x, b.y, b.z, b.w}};
-}
-__device__ __forceinline__ float dot8(const F8& a, const F8& b) {
-  float s0 = a.v[0] * b.v[0], s1 = a.v[1] * b.v[1];
-#pragma unroll
-  for (int i = 2; i < 8; i += 2) s0 = fmaf(a.v[i], b.v[i], s0), s1 = fmaf(a.v[i + 1], b.v[i + 1], s1);
-  return s0 + s1;
-}
-
-template <int D, bool ROT, bool TRAIN, int NL>
-__global__ void __launch_bounds__(kBwd8Threads, HV_BWD8_CTAS) rq_bwd_smem8_kernel(RqBwdArgs a) {
-  constexpr int LPR = D / 8;
-  constexpr int ROWS_PER_WARP = 32 / LPR;
-  constexpr bool rot = ROT && TRAIN;
-  extern __shared__ __align__(16) float s_cb[];  // [NL][K][D]
-  {
-    const int total4 = NL * a.k * (D / 4);
-    for (int i = threadIdx.x; i < total4; i += kBwd8Threads)
-      reinterpret_cast<float4*>(s_cb)[i] = __ldg(reinterpret_cast<const float4*>(a.codebooks) + i);
-  }
-  __syncthreads();
-
-  const int64_t lkd = static_cast<int64_t>(NL) * a.k * D;
-  const int lane = threadIdx.x & 31;
-  const int sub = lane % LPR;
-  const int warp_global = ptx::uniform((blockIdx.x * kBwd8Threads + threadIdx.x) >> 5);  // (see ptx::warp_index)
-  const int n_warps = (gridDim.x * kBwd8Threads) >> 5;
-  const int64_t n_groups = (a.n + ROWS_PER_WARP - 1) / ROWS_PER_WARP;
-  float* gc_base = a.n_replicas > 0 ? a.replicas + static_cast<int64_t>(blockIdx.x % a.n_replicas) * lkd : a.g_codebooks;
-
-  // the next iteration's inputs
-  F8 nx, nge[NL];
-  int nid[NL];
-  float ngl;
-  auto fetch = [&](int64_t g) {
-    const int64_t row = g * ROWS_PER_WARP + lane / LPR;
-    const int64_t rrow = row < a.n ? row : 0;  // keep every lane in the shuffles; the stores are masked
-    nx = ldg8<D>(a.x + rrow * D + sub * 4);
-    ngl = a.g_loss != nullptr ? __ldg(a.g_loss + rrow * a.g_loss_stride) : 0.f;
-#pragma unroll
-    for (int l = 0; l < NL; ++l) {
-      int64_t code = __ldg(a.ids + rrow * a.ids_row_stride + l * a.ids_level_stride);
-      code = code < 0 ? 0 : (code >= a.k ? a.k - 1 : code);
-      nid[l] = static_cast<int>(code);
-      if (a.g_emb != nullptr) {
-        nge[l] = ldg8<D>(a.g_emb + l * a.g_emb_level_stride + rrow * a.g_emb_row_stride + sub * 4);
-      } else {
-#pragma unroll
-        for (int i = 0; i < 8; ++i) nge[l].v[i] = 0.f;
-      }
-    }
-  };
-  if (warp_global < n_groups) fetch(warp_global);
-
-  for (int64_t g = warp_global; g < n_groups; g += n_warps) {
-    const int64_t row = g * ROWS_PER_WARP + lane / LPR;
-    const bool valid = row < a.n;
-    F8 r = nx;
-    const float gl = ngl;
-    F8 GE[NL];
-    const float* code_row[NL];
-#pragma unroll
-    for (int l = 0; l < NL; ++l) GE[l] = nge[l], code_row[l] = s_cb + (static_cast<int64_t>(l) * a.k + nid[l]) * D + sub * 4;
-    int id[NL];
-#pragma unroll
-    for (int l = 0; l < NL; ++l) id[l] = nid[l];
-    if (g + n_warps < n_groups) fetch(g + n_warps);
-
-    F8 R[NL];
-    float inv_r[NL], inv_e[NL], inv_s[NL];
-#pragma unroll
-    for (int l = 0; l < NL; ++l) {
-      const F8 e = lds8<D>(code_row[l]);
-      R[l] = r;
-      if (rot) {  // (same expressions as rq_bwd_kernel)
-        const float rr = group_sum<LPR>(dot8(r, r));
-        const float ee = group_sum<LPR>(dot8(e, e));
-        const float re = group_sum<LPR>(dot8(r, e));
-        const float ir = fast_inv_norm_eps(rr, 1e-8f);
-        const float ie = fast_inv_norm_eps(ee, 1e-8f);
-        const float ru = rr * ir;
-        const float rq = re * ie;
-        const float ss = fmaf(2.0f * rq, ir, fmaf(ru, ir, ee * ie * ie));  // |u + q|^2 from the three row sums
-        const float rs = ru + rq;
-        const float is = fast_inv_norm_floor(ss, 1e-6f);
-        inv_r[l] = ir, inv_e[l] = ie, inv_s[l] = is;
-        const float a2 = 2.0f * rs * is * is, b2 = 2.0f * ru;
-        const float cr = 1.0f - a2 * ir, ce = (b2 - a2) * ie;
-#pragma unroll
-        for (int i = 0; i < 8; ++i) r.v[i] -= fmaf(cr, r.v[i], ce * e.v[i]);
-      } else {
-#pragma unroll
-        for (int i = 0; i < 8; ++i) r.v[i] -= e.v[i];
-      }
-    }
-
-    F8 G;
-#pragma unroll
-    for (int i = 0; i < 8; ++i) G.v[i] = 0.f;
-    const float c2 = 2.0f * gl, cb2 = a.beta * c2;
-#pragma unroll
-    for (int l = NL - 1; l >= 0; --l) {
-      const F8 el = lds8<D>(code_row[l]);
-      const F8& rl = R[l];
-      F8 h, diff, ge_code;
-#pragma unroll
-      for (int i = 0; i < 8; ++i) {
-        h.v[i] = GE[l].v[i] - G.v[i];
-        diff.v[i] = rl.v[i] - el.v[i];
-        ge_code.v[i] = -c2 * diff.v[i];
-      }
-      if (TRAIN) {
-        if (rot) {
-          const float ir = inv_r[l], ie = inv_e[l], is = inv_s[l];
-          F8 u, q, w;
-#pragma unroll
-          for (int i = 0; i < 8; ++i) {
-            u.v[i] = rl.v[i] * ir;
-            q.v[i] = el.v[i] * ie;
-            w.v[i] = (u.v[i] + q.v[i]) * is;
-          }
-          const float hw2 = 2.0f * group_sum<LPR>(dot8(h, w));
-          const float hq2 = 2.0f * group_sum<LPR>(dot8(h, q));
-#pragma unroll
-          for (int i = 0; i < 8; ++i) h.v[i] = h.v[i] - hw2 * w.v[i] + hq2 * u.v[i];
-        }
-#pragma unroll
-        for (int i = 0; i < 8; ++i) G.v[i] += h.v[i] + cb2 * diff.v[i];
-      } else {
-#pragma unroll
-        for (int i = 0; i < 8; ++i) {
-          G.v[i] += cb2 * diff.v[i];
-          ge_code.v[i] += h.v[i];
-        }
-      }
-      if (valid) {
-        float* gc = gc_base + (static_cast<int64_t>(l) * a.k + id[l]) * D + sub * 4;
-        red_add_v4(gc, make_float4(ge_code.v[0], ge_code.v[1], ge_code.v[2], ge_code.v[3]));
-        red_add_v4(gc + D / 2, make_float4(ge_code.v[4], ge_code.v[5], ge_code.v[6], ge_code.v[7]));
-      }
-    }
-    if (valid) {
-      float* gx = a.g_x + row * D + sub * 4;
-      *reinterpret_cast<float4*>(gx) = make_float4(G.v[0], G.v[1], G.v[2], G.v[3]);
-      *reinterpret_cast<float4*>(gx + D / 2) = make_float4(G.v[4], G.v[5], G.v[6], G.v[7]);
-    }
-  }
-}
-
-// shapes the shared-memory variant serves: exact-level instantiation, codebooks within 96 KB, no per-level loss gradient,
-// and enough rows for 2 persistent CTAs per SM to amortise staging the codebooks
-#ifndef HV_BWD_SMEM_MIN_N
-#define HV_BWD_SMEM_MIN_N 65536
-#endif
+// shapes the shared-memory kernel serves: exact-level instantiation, codebooks within 96 KB, no per-level loss gradient,
+// and enough rows to amortise staging the codebooks
 template <int D>
 bool bwd_smem_ok(const RqBwdArgs& a) {
-  return (D == 16 || D == 32 || D == 64) && a.n_levels >= 1 && a.n_levels <= 4 && a.g_level_loss == nullptr && a.n >= HV_BWD_SMEM_MIN_N &&
-         static_cast<int64_t>(a.n_levels) * a.k * D * 4 <= kBwd2SmemLimit;
+  return (D == 16 || D == 32 || D == 64) && a.n_levels >= 1 && a.n_levels <= 4 && a.g_level_loss == nullptr && a.n >= kSmemMinRows &&
+         static_cast<int64_t>(a.n_levels) * a.k * D * 4 <= kSmemLimit;
 }
 
 template <int D>
@@ -529,40 +352,28 @@ int launch_d(const RqBwdArgs& a, bool rot, cudaStream_t stream) {
   int64_t ctas = (a.n + rows_per_cta - 1) / rows_per_cta;
   const int64_t cap = static_cast<int64_t>(props.sm_count) * 16;
   if (ctas > cap) ctas = cap;
-  auto go = [&](auto kernel) -> int {
-    kernel<<<static_cast<unsigned>(ctas), kBwdThreads, 0, stream>>>(a);
+  using Kernel = void (*)(RqBwdArgs);
+  auto go = [&](Kernel kernel, int64_t grid, int threads, int smem_bytes) -> int {
+    if (smem_bytes > 0) {
+      if (int st = prepare_kernel(kernel, 0, smem_bytes)) return st;
+    }
+    kernel<<<static_cast<unsigned>(grid), threads, smem_bytes, stream>>>(a);
     HV_CUDA_CHECK(cudaGetLastError());
     return HV_OK;
   };
   const bool train = a.training != 0;
   const bool r = rot && train;  // eval: the rotation plays no part
-  const bool smem_variant = bwd_smem_ok<D>(a);
-  const int smem_bytes = a.n_levels * a.k * D * 4;
-  auto go2 = [&](auto kernel) -> int {
-    if (int st = prepare_kernel(kernel, 0, smem_bytes)) return st;
-    kernel<<<HV_BWD2_CTAS * props.sm_count, kBwd2Threads, smem_bytes, stream>>>(a);
-    HV_CUDA_CHECK(cudaGetLastError());
-    return HV_OK;
-  };
-  auto go8 = [&](auto kernel) -> int {
-    if (int st = prepare_kernel(kernel, 0, smem_bytes)) return st;
-    kernel<<<HV_BWD8_CTAS * props.sm_count, kBwd8Threads, smem_bytes, stream>>>(a);
-    HV_CUDA_CHECK(cudaGetLastError());
-    return HV_OK;
-  };
   auto pick = [&](auto nl) -> int {
     constexpr int NLc = decltype(nl)::value;
     if constexpr (NLc > 0 && (D == 16 || D == 32 || D == 64)) {
-      if (smem_variant) {
-#ifndef HV_BWD_NO_LPR8
-        if (r) return go8(rq_bwd_smem8_kernel<D, true, true, NLc>);  // the rotation-trick chain is the instruction-bound one
-#endif
-        if (r) return go2(rq_bwd_smem_kernel<D, true, true, NLc>);
-        return train ? go2(rq_bwd_smem_kernel<D, false, true, NLc>) : go2(rq_bwd_smem_kernel<D, false, false, NLc>);
+      if (bwd_smem_ok<D>(a)) {  // eight floats per lane for the rotation trick in training, four for STE and eval
+        const Kernel k = r ? rq_bwd_smem_kernel<D, 8, true, true, NLc>
+                           : train ? rq_bwd_smem_kernel<D, 4, false, true, NLc> : rq_bwd_smem_kernel<D, 4, false, false, NLc>;
+        return go(k, props.sm_count, r ? kSmemThreads<8> : kSmemThreads<4>, a.n_levels * a.k * D * 4);
       }
     }
-    if (r) return go(rq_bwd_kernel<D, true, true, NLc>);
-    return train ? go(rq_bwd_kernel<D, false, true, NLc>) : go(rq_bwd_kernel<D, false, false, NLc>);
+    const Kernel k = r ? rq_bwd_kernel<D, true, true, NLc> : train ? rq_bwd_kernel<D, false, true, NLc> : rq_bwd_kernel<D, false, false, NLc>;
+    return go(k, ctas, kBwdThreads, 0);
   };
   if constexpr (D == 16 || D == 32 || D == 64) {  // the shipped shapes get exact-level instantiations
     switch (a.n_levels) {

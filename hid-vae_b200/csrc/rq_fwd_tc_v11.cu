@@ -41,18 +41,11 @@ namespace {
 
 using namespace rows;
 
-#ifndef HV_V11_WGS
-#define HV_V11_WGS 3  // measured: three owners at 128 registers beat four at 112 (spills)
-#endif
-constexpr int kWGs = HV_V11_WGS;  // row tiles in flight per CTA (owner warpgroups)
+constexpr int kWGs = 3;  // row tiles in flight per CTA (owner warpgroups); measured: three owners at 128 registers beat four at 112 (spills)
 constexpr int kIssuerWarp = kWGs * 4;   // the warp after the owners issues every tcgen05.mma
 constexpr int kThreads = (kWGs + 1) * 128;  // (register allocation is per warpgroup: the issuer's three siblings idle)
-// four owners: launch 96, owners take 112, the issuer's warpgroup keeps 24; three owners: 128 for everybody
-#ifndef HV_V11_OWNER_REGS
-#define HV_V11_OWNER_REGS 128
-#endif
 constexpr int kLaunchRegs = (65536 / kThreads) / 8 * 8;
-constexpr int kOwnerRegs = kWGs == 4 ? 112 : HV_V11_OWNER_REGS, kIssuerRegs = kWGs == 4 ? 24 : (HV_V11_OWNER_REGS > 128 ? 24 : 128);
+constexpr int kOwnerRegs = 128, kIssuerRegs = 128;  // three owners: 128 for everybody
 static_assert(kWGs * 128 * kOwnerRegs + 128 * kIssuerRegs <= kThreads * kLaunchRegs, "register hand-over must stay inside the launch allocation");
 constexpr int kTmemCols = 512;  // 3 x 128 accumulator columns + 4 x 32 A columns
 #ifdef HV_TC_INSTRUMENT
@@ -60,15 +53,6 @@ constexpr bool kInstr = true;
 #else
 constexpr bool kInstr = false;
 #endif
-
-// Scan of this thread's row over the 128 columns of one accumulator (rq_rows.cuh); -DHV_V11_SCAN=0: the unpipelined 16-column form
-__device__ __forceinline__ void scan_unit(uint32_t t0, float& m_out, int& col_out) {
-#if defined(HV_V11_SCAN) && HV_V11_SCAN == 0
-  scan_unit_x16(t0, m_out, col_out);
-#else
-  scan_unit_x8_pairs(t0, m_out, col_out);
-#endif
-}
 
 struct V11Params {
   const uint8_t* images;  // [L] packed bf16 images
@@ -199,11 +183,7 @@ __global__ void __launch_bounds__(kThreads, 1) rq_fwd_tc_v11_kernel(RqFwdArgs a,
         if (s < static_cast<uint32_t>(kWGs * n_levels)) ptx::mbar_wait(ptx::smem_u32(&bar_b_full[l]), 0u);  // images are loaded once
         issue(rwg, l, 0u);
         if (have_pending) issue(pend_wg, pend_l, 1u);
-#ifdef HV_V11_NO_DEFER
-        issue(rwg, l, 1u);
-#else
         have_pending = true, pend_wg = rwg, pend_l = l;
-#endif
       }
       if (have_pending) issue(pend_wg, pend_l, 1u);
     }
@@ -226,13 +206,11 @@ __global__ void __launch_bounds__(kThreads, 1) rq_fwd_tc_v11_kernel(RqFwdArgs a,
   for (int i = wg; i < my_tiles; i += kWGs) {
     const int64_t grow = tile_row0(i) + t;
     const bool valid = grow < a.n;
-#ifndef HV_V11_NO_PREFETCH
     if (q == 0 && lane == 0 && i + kWGs < my_tiles) {  // pull the warpgroup's next tile into L2
       const int64_t next0 = tile_row0(i + kWGs);
       const int64_t rows = a.n - next0 < kTileRows ? a.n - next0 : kTileRows;
       ptx::bulk_prefetch_l2(a.x + next0 * D, static_cast<uint32_t>(rows * D * 4));
     }
-#endif
     stamp(1);
     if (!have_x) load_x(i);
     have_x = false;
@@ -280,7 +258,7 @@ __global__ void __launch_bounds__(kThreads, 1) rq_fwd_tc_v11_kernel(RqFwdArgs a,
         stamp(u == 0 ? 5 : 9);
         float m;
         int c;
-        scan_unit(tmem_base + acc * kUnitCols + lane_bits, m, c);
+        scan_unit_x8_pairs(tmem_base + acc * kUnitCols + lane_bits, m, c);
         if (u == 0) stamp(8);
         ptx::tc_fence_before_sync();
         __syncwarp();

@@ -1,7 +1,7 @@
 // Building blocks of the row-owner kernel of the fused quantiser forward (rq_fwd_tc_v11.cu): D = 32, K <= 256, one 256-code
 // operand image per level resident in shared memory, a level = two units of 128 codes on 128-column accumulators in tensor
-// memory, A operand (the residual's bf16 hi | lo halves) in tensor memory.  The argmax scans, the MMA issue of one unit and
-// the bf16 split live here so that A/B builds of the kernel (tools/build_variant.sh) differ in one line.
+// memory, A operand (the residual's bf16 hi | lo halves) in tensor memory: the argmax scan, the MMA issue of one unit and the
+// bf16 split.  The streamed generation (rq_fwd_tc_v4.cu) scans its 256-column units with the same fold.
 //
 // Measured on B200 (tools/micro/tmem_ld_shapes.cu): max.f32 with two inputs issues at 3.9 warp-instructions / cycle / SM,
 // with three inputs at 1.95 -- a 3-input maximum costs the ALU pipe as much as two 2-input ones and only saves the issue
@@ -34,12 +34,6 @@ __device__ __forceinline__ float max3(float a, float b, float c) {
   return d;
 }
 __device__ __forceinline__ float f(uint32_t v) { return __uint_as_float(v); }
-__device__ __forceinline__ float max16(const uint32_t (&v)[16]) {
-  const float a0 = max3(f(v[0]), f(v[1]), f(v[2])), a1 = max3(f(v[3]), f(v[4]), f(v[5]));
-  const float a2 = max3(f(v[6]), f(v[7]), f(v[8])), a3 = max3(f(v[9]), f(v[10]), f(v[11]));
-  const float a4 = max3(f(v[12]), f(v[13]), f(v[14]));
-  return fmaxf(max3(a0, a1, a2), max3(a3, a4, f(v[15])));
-}
 __device__ __forceinline__ float max8(const uint32_t (&v)[8]) {
   return max3(max3(f(v[0]), f(v[1]), f(v[2])), max3(f(v[3]), f(v[4]), f(v[5])), fmaxf(f(v[6]), f(v[7])));
 }
@@ -64,54 +58,6 @@ __device__ __forceinline__ void scan_chunk_exact(const uint32_t (&v)[W], int bas
 // and its FIRST column.  Fast path: a 2-D fold -- maxima per column class (column mod W) and per chunk (column / W) --
 // locates the maximiser when exactly one class and one chunk attain it; otherwise the warp re-reads the unit and takes the
 // exact first-index path.
-
-// Two 16-column loads per step, 3-input maxima (1.0 ALU instruction per score); the load latency is exposed four times.
-__device__ __forceinline__ void scan_unit_x16(uint32_t t0, float& m_out, int& col_out) {
-  float g[16], cm[8];
-  uint32_t a[16], b[16];
-#pragma unroll
-  for (int p = 0; p < 4; ++p) {
-    ptx::tmem_ld_32x16(t0 + 32 * p, a);
-    ptx::tmem_ld_32x16(t0 + 32 * p + 16, b);
-    ptx::tmem_wait_ld(a, b);
-    cm[2 * p] = max16(a);
-    cm[2 * p + 1] = max16(b);
-#pragma unroll
-    for (int j = 0; j < 16; ++j) g[j] = p == 0 ? fmaxf(f(a[j]), f(b[j])) : max3(g[j], f(a[j]), f(b[j]));
-  }
-  const float m = max3(max3(cm[0], cm[1], cm[2]), max3(cm[3], cm[4], cm[5]), fmaxf(cm[6], cm[7]));
-  // class of the maximiser: sum_j [g_j == m] * (32 + j);  chunk: sum_c [cm_c == m] * (16 + c)   (FMA pipe)
-  float s4[4] = {0.f, 0.f, 0.f, 0.f};
-#pragma unroll
-  for (int j = 0; j < 16; ++j) {
-    const float e = __saturatef(fmaf(g[j] - m, kBig, 1.0f));
-    s4[j & 3] = fmaf(e, static_cast<float>(32 + j), s4[j & 3]);
-  }
-  float c2[2] = {0.f, 0.f};
-#pragma unroll
-  for (int c = 0; c < 8; ++c) {
-    const float e = __saturatef(fmaf(cm[c] - m, kBig, 1.0f));
-    c2[c & 1] = fmaf(e, static_cast<float>(16 + c), c2[c & 1]);
-  }
-  const float cls = (s4[0] + s4[1]) + (s4[2] + s4[3]);
-  const float chk = c2[0] + c2[1];
-  // exactly one class and one chunk attain m (all-padding units, m = -1e30, cannot win anyway; NaN takes the exact path)
-  const bool unique = (cls < 64.f && chk < 32.f) || m < -1e29f;
-  float best = m;
-  int col = 16 * (static_cast<int>(chk) - 16) + static_cast<int>(cls) - 32;
-  if (__any_sync(0xffffffffu, !unique)) {
-    best = -INFINITY;
-    col = 0;
-#pragma unroll 1
-    for (int c = 0; c < 8; ++c) {
-      ptx::tmem_ld_32x16(t0 + 16 * c, a);
-      ptx::tmem_wait_ld16(a);
-      scan_chunk_exact<16>(a, 16 * c, best, col);
-    }
-  }
-  m_out = best;
-  col_out = col;
-}
 
 // Location of the maximiser from the fold over 8 classes x NC chunks (shared by the 8-column scans).
 template <int NC>
@@ -159,8 +105,9 @@ __device__ __forceinline__ void locate_8(uint32_t t0, const float (&g)[8], const
 }
 
 // 8-column loads over 8 NC columns from `t0`, software-pipelined: while one pair of loads is processed (3-input maxima,
-// 1.0 ALU instruction per score) the next pair is in flight.  Same 32 load registers as scan_unit_x16 and no spills beside
-// the 32-float row (the x16 form spills 20 bytes): 4 Mi-row encode 0.609 -> 0.587 ms, training forward 0.927 -> 0.852 ms.
+// 1.0 ALU instruction per score) the next pair is in flight.  It takes the same 32 load registers as an unpipelined scan of
+// two 16-column loads per step and spills nothing beside the 32-float row (that scan spilled 20 bytes and exposed the load
+// latency four times per unit): 4 Mi-row encode 0.609 -> 0.587 ms, training forward 0.927 -> 0.852 ms.
 template <int NC>
 __device__ __forceinline__ void scan_x8_pairs(uint32_t t0, float& m_out, int& col_out) {
   float g[8], cm[NC];

@@ -270,8 +270,8 @@ def test_backward_vs_oracle_autograd(ops, algo, mname, training, shape):
 @pytest.mark.parametrize("shape", [(65536 + 77, 32, 256, 3), (70001, 64, 128, 2), (66000, 16, 512, 3)],
                          ids=lambda s: "n%d_d%d_k%d_L%d" % s)
 def test_backward_large_n_variant_equals_row_kernel(ops, mname, training, shape):
-    """From 65,536 rows on (codebooks within 96 KB) the backward runs its shared-memory / prefetching variant
-    (rq_bwd_smem_kernel; rq_bwd_smem8_kernel for the rotation trick).  The same rows in two calls below that size run the
+    """From 65,536 rows on (codebooks within 96 KB) the backward runs its shared-memory / prefetching kernel
+    (rq_bwd_smem_kernel: four floats per lane, eight for the rotation trick).  The same rows in two calls below that size run the
     row kernel, which the oracle tests above pin: g_x must be bit-identical where the per-row expressions are the same, and
     equal up to the order of the row sums (eight floats per lane instead of four) for the rotation-trick kernel -- with the
     bar of the oracle comparison; the codebook gradient equal up to the order of the sums."""
@@ -300,8 +300,8 @@ def test_backward_large_n_variant_equals_row_kernel(ops, mname, training, shape)
 @pytest.mark.parametrize("mname", ["ste", "rot"])
 @pytest.mark.parametrize("shape", [(65536 + 77, 32, 256, 3), (66001, 64, 128, 2)], ids=lambda s: "n%d_d%d_k%d_L%d" % s)
 def test_backward_large_n_variant_vs_oracle_autograd(ops, mname, shape):
-    """The shared-memory backward kernels (from 65,536 rows on) against the oracle's autograd directly, on the oracle's own
-    ids (so that no near-tie row can follow another code)."""
+    """The shared-memory backward kernel (from 65,536 rows on; four floats per lane, eight for the rotation trick) against
+    the oracle's autograd directly, on the oracle's own ids (so that no near-tie row can follow another code)."""
     n, d, k, L = shape
     beta = 0.4
     x = unit_rows(n, d, seed=61)

@@ -32,7 +32,7 @@ ALGO = {
     "encoder": ("enc_mlp_kernel, 1 Mi rows of 768-d items -> z [N, 32]", 1 << 20, (1 << 20) * (4 * 768 + 4 * 32)),
     "rq_encode": ("rq_fwd_tc_v11_kernel<0,0> ids only, 4 Mi rows D32 K256 L3", 1 << 22, (1 << 22) * (4 * 32 + 8 * 3)),
     "train_fwd": ("rq_fwd_tc_v11_kernel<rot,out> emb_out + loss + ids, 4 Mi rows", 1 << 22, (1 << 22) * (4 * 32 + 4 * 32 * 3 + 8 * 3 + 4)),
-    "train_bwd": ("rq_bwd_smem8_kernel<32,rot,train,3>, 4 Mi rows", 1 << 22, (1 << 22) * (4 * 32 + 8 * 3 + 4 * 32 * 3 + 4 + 4 * 32) + 4 * 3 * 256 * 32),
+    "train_bwd": ("rq_bwd_smem_kernel<32,8,rot,train,3>, 4 Mi rows", 1 << 22, (1 << 22) * (4 * 32 + 8 * 3 + 4 * 32 * 3 + 4 + 4 * 32) + 4 * 3 * 256 * 32),
     "c4": ("large-codebook encode 65,536 x D64 x K4096 x L4", 65536, 65536 * (4 * 64 + 8 * 4) + 4 * 4096 * (4 * 64 + 32) * 4),
     "kmeans": ("kmeans_segsum_kernel<64>, 65,536 rows, K 4096", 65536, 65536 * (4 * 64 + 12) + 4096 * 65 * 4),
     "uniq": ("uniq_sorted_kernel, 65,536 rows of 3 ids + 32-d features (every row has a twin)", 65536, 65536 * (8 * 3 + 12 + 4 * 32)),

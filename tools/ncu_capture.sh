@@ -19,7 +19,7 @@ cap() {  # name, workload of run_kernels_once.py, kernel regex, launches to skip
 cap encoder   encoder 'enc_mlp_kernel'       1 "--import-source on"
 cap rq_encode rq      'rq_fwd_tc_v11_kernel' 1 "--import-source on"
 cap train_fwd train   'rq_fwd_tc_v11_kernel' 1 ""
-cap train_bwd train   'rq_bwd_smem8_kernel'  1 "--import-source on"
+cap train_bwd train   'rq_bwd_smem_kernel'   1 "--import-source on"
 cap c4        c4      'rq_fwd_tc'            1 "--import-source on"
 cap kmeans    aux     'kmeans_segsum_kernel' 0 ""
 cap uniq      aux     'uniq_sorted_kernel'   0 ""
