@@ -276,7 +276,7 @@ __global__ void __launch_bounds__(kThreads) gumbel_bwd_kernel(GumbelArgs a) {
       const float gl = a.g_loss != nullptr ? __ldg(a.g_loss + row) : 0.f;
       float x[D], ge[D];
       load_row<D>(x, a.x + row * D);
-      float gee = 0.f;
+      float gee;
       {
         float eo[D];
         load_row<D>(eo, a.emb_out + row * D);
@@ -287,10 +287,10 @@ __global__ void __launch_bounds__(kThreads) gumbel_bwd_kernel(GumbelArgs a) {
           for (int d = 0; d < D; ++d) ge[d] = 0.f;
         }
 #pragma unroll
-        for (int d = 0; d < D; ++d) {
-          ge[d] = fmaf(2.0f * gl, eo[d] - x[d], ge[d]);  // + d emb_loss / d emb (modules/loss.py:42)
-          gee = fmaf(ge[d], eo[d], gee);
-        }
+        for (int d = 0; d < D; ++d) ge[d] = fmaf(2.0f * gl, eo[d] - x[d], ge[d]);  // + d emb_loss / d emb (modules/loss.py:42)
+        // in the summation order of ge.c_k below: where emb equals a code bit for bit (K = 1, or a softmax that underflowed to
+        // one-hot at low T) its a_k is then exactly 0, as in exact arithmetic, instead of fp32 noise amplified by 1 / T
+        gee = dot_row<D>(ge, eo);
       }
       const float xx = dot_row<D>(x, x);
       const float lse = __ldg(a.lse + row);
