@@ -173,4 +173,37 @@ int hv_rq_forward(const float* x, int64_t n, int d, const float* codebooks, int 
   }
 }
 
+size_t hv_semid_dedup_workspace_bytes(int64_t rows) { return hv::semid_dedup_workspace_bytes(rows); }
+
+int hv_semid_dedup(const int64_t* ids, int64_t rows, int64_t width, int64_t row_stride, int64_t col_stride, int bits,
+                   const int64_t* prior_keys, const int64_t* prior_counts, int64_t n_prior, int64_t* digits, int64_t digit_stride,
+                   int64_t* run_keys, int64_t* run_counts, int64_t* stats, void* workspace, size_t workspace_bytes, void* stream) {
+  using namespace hv;
+  if (rows < 0 || width <= 0 || bits <= 0 || n_prior < 0) {
+    set_error("hv_semid_dedup: bad shape rows=%lld width=%lld bits=%d n_prior=%lld", (long long)rows, (long long)width, bits,
+              (long long)n_prior);
+    return HV_ERR_BAD_SHAPE;
+  }
+  if (width > 63 || bits > 63 || width * bits > 63) {
+    set_error("hv_semid_dedup: width * bits = %lld exceeds the 63 bits of an exact key", (long long)width * bits);
+    return HV_ERR_UNSUPPORTED;
+  }
+  if (rows >= kSemidDedupMaxRows) {
+    set_error("hv_semid_dedup: %lld rows, at most 2^31 - 1 per call", (long long)rows);
+    return HV_ERR_UNSUPPORTED;
+  }
+  if (!stats || (rows > 0 && (!ids || !digits || !run_keys || !run_counts)) || (n_prior > 0 && (!prior_keys || !prior_counts))) {
+    set_error("hv_semid_dedup: ids, digits, run_keys, run_counts, stats (and prior_keys / prior_counts when n_prior > 0) must be non-null");
+    return HV_ERR_NULL;
+  }
+  if (rows > 0 && (workspace == nullptr || workspace_bytes < semid_dedup_workspace_bytes(rows))) {
+    set_error("hv_semid_dedup: workspace of %zu bytes, hv_semid_dedup_workspace_bytes(%lld) = %zu needed", workspace ? workspace_bytes : 0,
+              (long long)rows, semid_dedup_workspace_bytes(rows));
+    return HV_ERR_WORKSPACE;
+  }
+  SemidDedupArgs a{ids, rows, width, row_stride, col_stride, bits, prior_keys, prior_counts, n_prior, digits, digit_stride,
+                   run_keys, run_counts, stats};
+  return launch_semid_dedup(a, workspace, workspace_bytes, static_cast<cudaStream_t>(stream));
+}
+
 }  // extern "C"

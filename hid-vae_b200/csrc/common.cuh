@@ -75,6 +75,24 @@ bool rq_fwd_tc_supported(int d, int k, int n_levels);
 size_t rq_fwd_tc_workspace_bytes(int d, int k, int n_levels);
 size_t rq_bwd_workspace_bytes(int64_t n, int d, int k, int n_levels);
 
+// Collision digit of semantic-ID tuples (semid_dedup.cu); arguments are those of hv_semid_dedup, validated by it.
+struct SemidDedupArgs {
+  const int64_t* ids;
+  int64_t rows, width, row_stride, col_stride;
+  int bits;
+  const int64_t* prior_keys;
+  const int64_t* prior_counts;
+  int64_t n_prior;
+  int64_t* digits;
+  int64_t digit_stride;
+  int64_t* run_keys;
+  int64_t* run_counts;
+  int64_t* stats;
+};
+constexpr int64_t kSemidDedupMaxRows = 1ll << 31;  // row indices travel as uint32 with a flag bit; cub takes an int count
+size_t semid_dedup_workspace_bytes(int64_t rows);
+int launch_semid_dedup(const SemidDedupArgs& a, void* workspace, size_t workspace_bytes, cudaStream_t stream);
+
 // 1 / (sqrt(v) + eps) and 1 / max(sqrt(v), floor) on the special-function unit: sqrt.approx (max relative error 2^-23) and
 // rcp.approx followed by one Newton step (the reciprocal is then correctly rounded up to the last bit of its argument).
 // 6 instructions instead of the ~16 + slow-path branches of an IEEE sqrt and division; three of these per row and level.

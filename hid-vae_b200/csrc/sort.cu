@@ -1,5 +1,7 @@
-// cub::DeviceRadixSort behind sort.cuh (the one CUB instantiation of the library: 64-bit keys, 32-bit row indices).
+// cub::DeviceRadixSort and cub::DeviceScan behind sort.cuh (the library's two CUB instantiations: a radix sort of 64-bit keys
+// with 32-bit row indices, and an in-place inclusive sum of 64-bit words).
 #include <cub/device/device_radix_sort.cuh>
+#include <cub/device/device_scan.cuh>
 
 #include "sort.cuh"
 
@@ -43,6 +45,19 @@ int sort_pairs(const SortBuffers& b, int64_t n, int end_bit, cudaStream_t stream
   size_t bytes = b.temp_bytes;
   HV_CUDA_CHECK(cub::DeviceRadixSort::SortPairs(b.temp, bytes, b.keys_in, b.keys_out, b.vals_in, b.vals_out, static_cast<int>(n), 0,
                                                 end_bit, stream));
+  return HV_OK;
+}
+
+size_t scan_temp_bytes(int64_t n) {
+  if (n <= 0 || n >= (1ll << 31)) return 0;
+  size_t bytes = 0;
+  cub::DeviceScan::InclusiveSum(nullptr, bytes, static_cast<uint64_t*>(nullptr), static_cast<int>(n));
+  return bytes;
+}
+
+int inclusive_sum_u64(void* temp, size_t temp_bytes, uint64_t* data, int64_t n, cudaStream_t stream) {
+  size_t bytes = temp_bytes;
+  HV_CUDA_CHECK(cub::DeviceScan::InclusiveSum(temp, bytes, data, static_cast<int>(n), stream));
   return HV_OK;
 }
 

@@ -1,5 +1,6 @@
 // Stable key sort of row indices (cub::DeviceRadixSort on 64-bit keys) shared by the k-means update (sort rows by
-// cluster -> segmented sums) and the uniqueness loss (sort rows by id tuple -> runs of identical tuples).
+// cluster -> segmented sums), the uniqueness loss and the semantic-ID collision digit (sort rows by id tuple -> runs of
+// identical tuples); and the in-place 64-bit inclusive sum (cub::DeviceScan) that numbers those runs.
 // The library never allocates: the caller provides hv_sort_workspace_bytes(n) bytes.
 #pragma once
 
@@ -21,5 +22,10 @@ size_t sort_workspace_bytes(int64_t n);
 bool sort_carve(void* workspace, size_t workspace_bytes, int64_t n, SortBuffers* out);
 // keys_in / vals_in -> keys_out / vals_out, ascending, stable, bits [0, end_bit) of the key
 int sort_pairs(const SortBuffers& b, int64_t n, int end_bit, cudaStream_t stream);
+
+// temporary storage of inclusive_sum_u64 for n words (0 for n <= 0 or n >= 2^31)
+size_t scan_temp_bytes(int64_t n);
+// data[i] <- data[0] + ... + data[i], in place
+int inclusive_sum_u64(void* temp, size_t temp_bytes, uint64_t* data, int64_t n, cudaStream_t stream);
 
 }  // namespace hv

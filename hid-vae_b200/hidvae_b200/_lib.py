@@ -49,6 +49,9 @@ SIGNATURES = {
                                 c_void_p, c_void_p, c_size_t, c_void_p]),
     "hv_uniq_backward": (c_int, [c_void_p, c_int64, c_int64, c_int64, c_int64, c_void_p, c_int, c_float, c_float,
                                  c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
+    "hv_semid_dedup_workspace_bytes": (c_size_t, [c_int64]),
+    "hv_semid_dedup": (c_int, [c_void_p, c_int64, c_int64, c_int64, c_int64, c_int, c_void_p, c_void_p, c_int64, c_void_p,
+                               c_int64, c_void_p, c_void_p, c_void_p, c_void_p, c_size_t, c_void_p]),
     "hv_gumbel_supported": (c_int, [c_int, c_int]),
     "hv_gumbel_uniforms": (c_int, [c_int64, c_int, c_uint64, c_uint64, c_void_p, c_void_p]),
     "hv_gumbel_forward": (c_int, [c_void_p, c_int64, c_int, c_void_p, c_int, c_float, c_float, c_void_p, c_uint64, c_uint64,

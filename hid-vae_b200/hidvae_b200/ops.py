@@ -8,6 +8,7 @@ Mirrors, per function, the reference call sequence it replaces:
   encoder_pack / encoder_forward   modules/encoder.py:23-36 (the MLP in front of the quantiser, eval passes)
   kmeans_*                    init/kmeans.py:43-61
   uniqueness_loss / count     modules/h_rqvae.py:41-105, :645-648
+  semid_dedup / merge_runs    the collision digit of HSemanticIdTokenizer(use_dedup_dim=True)
 """
 from __future__ import annotations
 
@@ -436,3 +437,76 @@ def uniqueness_loss(ids: Tensor, feats: Tensor, margin: float, weight: float) ->
 def count_rows_with_later_twin(ids: Tensor) -> Tensor:
     """0-d double tensor: number of rows that have a LATER identical row; p_unique_ids = 1 - this / rows."""
     return uniq_stats(ids, None, 0.0)[2]
+
+
+# ------------------------------------------------------------------------------------------------------------------
+# semantic-ID collision digit (HSemanticIdTokenizer(use_dedup_dim=True))
+# ------------------------------------------------------------------------------------------------------------------
+class DedupResult(NamedTuple):
+    digits: Tensor      # [rows] int64: earlier rows (and prior rows) with the same tuple; -1 for a row with an id out of range
+    run_keys: Tensor    # [rows] int64 capacity: the call's distinct tuple keys, ascending; the first stats[0] are valid
+    run_counts: Tensor  # [rows] int64 capacity: rows of the call holding each key
+    stats: Tensor       # [3] int64: distinct tuples, largest digit (-1 if none), rows with an id outside [0, 2^bits)
+
+
+def dedup_bits(codebook_size: int) -> int:
+    """Bits of one id in the exact tuple key: ceil(log2 K), at least 1."""
+    return max(1, (int(codebook_size) - 1).bit_length())
+
+
+def dedup_key(ids: Tensor, bits: int) -> Tensor:
+    """The kernel's key of every tuple, in torch: sum_c ids[c] << bits * (width - 1 - c) (ids must lie in [0, 2^bits))."""
+    width = ids.shape[-1]
+    shifts = torch.arange(width - 1, -1, -1, device=ids.device, dtype=torch.int64) * int(bits)
+    return (ids.to(torch.int64) << shifts).sum(-1)
+
+
+def semid_dedup(ids: Tensor, bits: int, prior=None, digits_out: Optional[Tensor] = None) -> DedupResult:
+    """Collision digit of every row of `ids` [rows, width] (any strides): the number of earlier rows with the same tuple,
+    plus that tuple's count in `prior` = (keys, counts), the ascending keys of tuples seen before these rows and how often
+    (e.g. merge_runs of the lower ranks' run lists).  hv_semid_dedup: one stable radix sort of exact keys, no host sync.
+    `digits_out` (int64 [rows], any stride, e.g. column L of an [N, L + 1] table) receives the digits in place.
+    width * bits must be <= 63 (the key is exact); wider shapes raise ValueError."""
+    if ids.dtype != torch.int64 or ids.dim() != 2:
+        raise ValueError("semid_dedup: ids must be int64 [rows, width]")
+    rows, width = ids.shape
+    bits = int(bits)
+    if bits < 1 or width < 1 or width * bits > 63:
+        raise ValueError(f"semid_dedup: width {width} x {bits} bits does not fit an exact 63-bit key")
+    _require_cuda(ids)
+    dev = ids.device
+    digits = digits_out if digits_out is not None else torch.empty((rows,), dtype=torch.int64, device=dev)
+    if digits.dtype != torch.int64 or digits.shape != (rows,) or digits.device != dev:
+        raise ValueError("semid_dedup: digits_out must be int64 [rows] on the device of ids")
+    prior_keys = prior_counts = None
+    n_prior = 0
+    if prior is not None:
+        prior_keys, prior_counts = prior
+        _require_cuda(prior_keys, prior_counts)
+        prior_keys, prior_counts = prior_keys.to(torch.int64).contiguous(), prior_counts.to(torch.int64).contiguous()
+        n_prior = prior_keys.numel()
+        if prior_counts.numel() != n_prior:
+            raise ValueError("semid_dedup: prior keys and counts differ in length")
+    run_keys = torch.empty((rows,), dtype=torch.int64, device=dev)
+    run_counts = torch.empty((rows,), dtype=torch.int64, device=dev)
+    stats = torch.empty((3,), dtype=torch.int64, device=dev)
+    ws_bytes = int(lib.hv_semid_dedup_workspace_bytes(rows))
+    ws = torch.empty(ws_bytes, dtype=torch.uint8, device=dev) if ws_bytes else None
+    with torch.cuda.device(dev):
+        check(lib.hv_semid_dedup(ids.data_ptr(), rows, width, ids.stride(0), ids.stride(1), bits,
+                                 _ptr(prior_keys) if n_prior else None, _ptr(prior_counts) if n_prior else None, n_prior,
+                                 digits.data_ptr(), digits.stride(0), run_keys.data_ptr(), run_counts.data_ptr(),
+                                 stats.data_ptr(), _ptr(ws), ws_bytes, _stream(ids)))
+    return DedupResult(digits, run_keys, run_counts, stats)
+
+
+def merge_runs(runs):
+    """[(keys, counts), ...] -> (keys, counts): the union of run lists, ascending, with the counts of equal keys added."""
+    runs = list(runs)
+    if not runs:
+        raise ValueError("merge_runs: no run list given")
+    keys = torch.cat([k.reshape(-1).to(torch.int64) for k, _ in runs])
+    counts = torch.cat([c.reshape(-1).to(torch.int64) for _, c in runs])
+    keys, order = torch.sort(keys)
+    merged, inverse = torch.unique_consecutive(keys, return_inverse=True)
+    return merged, torch.zeros_like(merged).index_add_(0, inverse, counts[order])

@@ -7,7 +7,9 @@ concatenated / interleaved id modes the trainer uses -- runs encode + the L-leve
 `predict_tags`, and concatenates Python lists of small tensors (h_semids.py:109-195).  Here the catalogue is cut into
 large chunks; per chunk one encoder pass and ONE fused L-level kernel write the ids straight into their columns of
 the preallocated `cached_ids [N, L (+ L_tags)]` table, and the tag heads reuse that launch's per-level embeddings.
-`shard=(rank, world)` assigns a contiguous item range to every rank; `gather_shards` is the only collective.
+`shard=(rank, world)` assigns a contiguous item range to every rank; `gather_shards` is the only collective of the id table.
+With `use_dedup_dim` a last column numbers the items that share a semantic-id tuple (the TIGER-style collision digit,
+ops.semid_dedup); sharded, the ranks exchange only their lists of distinct tuples to make those digits global.
 """
 from typing import List, Optional, Tuple
 
@@ -60,6 +62,8 @@ class HSemanticIdTokenizer(nn.Module):
         super().__init__()
         if sum(map(bool, (use_dedup_dim, use_concatenated_ids, use_interleaved_ids))) > 1:
             raise ValueError("use_dedup_dim, use_concatenated_ids and use_interleaved_ids are mutually exclusive")
+        if use_dedup_dim and n_layers * ops.dedup_bits(codebook_size) > 63:
+            raise ValueError(f"use_dedup_dim: {n_layers} levels of {codebook_size} codes do not fit an exact 63-bit tuple key")
         # The reference sets torch.set_float32_matmul_precision('high') at import (modules/h_rqvae.py:21), i.e. TF32 encoder
         # GEMMs on a GPU.  encoder_precision (modules/encoder.py): "fused" = the one-kernel tcgen05 encoder with fp16
         # operands (the same 11-bit significand, fp32 accumulation); "tf32" / "fp32" = the PyTorch layers on cuBLAS
@@ -86,6 +90,13 @@ class HSemanticIdTokenizer(nn.Module):
 
     def reset(self) -> None:
         self.cached_ids = None
+        self._dedup_stats = None
+
+    @property
+    def dedup_stats(self) -> Optional[Tuple[int, int, int]]:
+        """(rows, distinct semantic-id tuples, largest collision digit) over the whole catalogue after
+        `precompute_corpus_ids` with `use_dedup_dim` (None otherwise).  The last id position takes largest digit + 1 values."""
+        return None if self._dedup_stats is None else tuple(int(v) for v in self._dedup_stats)
 
     def _get_hits(self, query: Tensor, key: Tensor) -> Tensor:
         return (key.unsqueeze(0) == query.unsqueeze(1)).all(dim=-1)
@@ -118,8 +129,10 @@ class HSemanticIdTokenizer(nn.Module):
 
     @torch.no_grad()
     @eval_mode
-    def precompute_corpus_ids(self, movie_dataset, shard: Optional[Tuple[int, int]] = None) -> Tensor:
-        """cached_ids [N, sem_ids_dim] int64 for the whole catalogue (or this rank's contiguous shard of it)."""
+    def precompute_corpus_ids(self, movie_dataset, shard: Optional[Tuple[int, int]] = None, process_group=None) -> Tensor:
+        """cached_ids [N, sem_ids_dim] int64 for the whole catalogue (or this rank's contiguous shard of it).  With
+        `use_dedup_dim`, column L holds every item's collision digit over the whole catalogue in item order, also on a
+        shard (the ranks of `process_group` exchange their distinct tuples), so `gather_shards` stays a concatenation."""
         model = self.hrq_vae
         dev = model.device
         n_total = movie_dataset.shape[0] if isinstance(movie_dataset, Tensor) else len(movie_dataset)
@@ -129,7 +142,7 @@ class HSemanticIdTokenizer(nn.Module):
             per = (n_total + world - 1) // world
             lo_all, hi_all = min(rank * per, n_total), min((rank + 1) * per, n_total)
         sem_cols, tag_cols = self._columns()
-        width = len(sem_cols) + len(tag_cols)
+        width = len(sem_cols) + len(tag_cols) + int(self.use_dedup_dim)
         table = torch.empty((hi_all - lo_all, width), dtype=torch.int64, device=dev)
         contiguous_sem = sem_cols == list(range(len(sem_cols)))
         codebooks = model.effective_codebooks().detach()
@@ -154,8 +167,38 @@ class HSemanticIdTokenizer(nn.Module):
                 if tags.shape[0] != ids.shape[0]:
                     raise ValueError(f"Semantic ID batch size ({ids.shape[0]}) does not match predicted tag batch size ({tags.shape[0]})")
                 rows[:, tag_cols] = tags
+        if self.use_dedup_dim:
+            world = shard[1] if shard is not None else 1
+            self._dedup_stats = self._assign_digits(table, n_total, shard[0] if world > 1 else 0, world, process_group)
         self.cached_ids = table
         return self.cached_ids
+
+    def _assign_digits(self, table: Tensor, n_total: int, rank: int, world: int, process_group) -> Tensor:
+        """table[:, L] <- collision digits of table[:, :L], in place; returns (rows, distinct, largest digit) of the catalogue.
+        Sharded: every rank sorts its shard once to get its distinct tuples, the run lists are all-gathered (16 B per
+        distinct tuple of each shard), and rank r sorts again with the merged lists of ranks < r as prior counts."""
+        L, bits = self.n_layers, ops.dedup_bits(self.codebook_size)
+        ids, digits = table[:, :L], table[:, L]
+        local = ops.semid_dedup(ids, bits, digits_out=digits)
+        if world == 1:
+            return torch.stack([torch.full_like(local.stats[0], n_total), local.stats[0], local.stats[1]])
+        import torch.distributed as dist
+        dev = table.device
+        sizes = [torch.zeros(1, dtype=torch.int64, device=dev) for _ in range(world)]
+        dist.all_gather(sizes, local.stats[:1].clone(), group=process_group)
+        sizes = [int(v) for v in sizes]
+        padded = torch.zeros((2, max(sizes)), dtype=torch.int64, device=dev)
+        padded[0, : sizes[rank]] = local.run_keys[: sizes[rank]]
+        padded[1, : sizes[rank]] = local.run_counts[: sizes[rank]]
+        parts = [torch.empty_like(padded) for _ in range(world)]
+        dist.all_gather(parts, padded, group=process_group)
+        lists = [(p[0, :n], p[1, :n]) for p, n in zip(parts, sizes)]
+        top = local.stats[1:2].clone()
+        if rank > 0:
+            top = ops.semid_dedup(ids, bits, prior=ops.merge_runs(lists[:rank]), digits_out=digits).stats[1:2].clone()
+        dist.all_reduce(top, op=dist.ReduceOp.MAX, group=process_group)
+        distinct = ops.merge_runs(lists)[0].numel()
+        return torch.tensor([n_total, distinct, int(top)], dtype=torch.int64)
 
     def gather_shards(self, process_group=None) -> Tensor:
         """all_gather of every rank's shard of `cached_ids` (the only collective of bulk assignment)."""

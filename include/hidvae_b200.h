@@ -162,6 +162,31 @@ int hv_uniq_backward(const int64_t* ids, int64_t rows, int64_t width, int64_t ro
                      const float* g_out, float* g_feats, void* workspace, size_t workspace_bytes, void* stream);
 
 /*
+ * Collision digit of semantic-ID tuples: the trailing id position of HSemanticIdTokenizer(use_dedup_dim=True), which
+ * makes every item's id unique.  Over `rows` tuples of `width` int64 ids (element (r, c) at ids[r*row_stride + c*col_stride]):
+ *   digit[r] = prior count of tuple r + #{ r' < r : tuple r' == tuple r }
+ * written to digits[r*digit_stride] (digit_stride = L + 1 writes column L of an [N, L + 1] table whose first L columns
+ * are `ids`).  Each tuple is packed into the exact key sum_c ids[c] << bits*(width-1-c), which ascends in lexicographic
+ * tuple order; width * bits must be <= 63, else HV_ERR_UNSUPPORTED.  Rows are key-sorted (stable radix sort over
+ * width*bits bits) and runs of equal keys are numbered by a scan: O(rows), whatever the number of repeats.
+ *   bits          >= 1, ceil(log2 K) for codebooks of K codes
+ *   prior_keys    [n_prior] ascending keys of tuples seen before these rows (e.g. the lower ranks' shards of a
+ *                 catalogue) with their counts prior_counts [n_prior]; NULL / 0 for none
+ *   run_keys, run_counts  [rows] capacity: the distinct keys of THIS call, ascending, and how many of its rows hold each
+ *                 (prior counts not included); the first stats[0] entries are valid
+ *   stats         [3] int64, OVERWRITTEN: number of distinct tuples, largest digit (-1 when there is none), number of rows
+ *                 with an id outside [0, 2^bits) -- those rows get digit -1 and belong to no run
+ *   workspace     hv_semid_dedup_workspace_bytes(rows) bytes (0 for rows = 0; 0 = unsupported for rows >= 2^31)
+ * Argument errors (bad shape, NULL, small workspace, width * bits > 63, rows >= 2^31) return before any CUDA call.  No
+ * allocation and no host synchronisation: CUDA-graph capturable.
+ */
+size_t hv_semid_dedup_workspace_bytes(int64_t rows);
+int hv_semid_dedup(const int64_t* ids, int64_t rows, int64_t width, int64_t row_stride, int64_t col_stride, int bits,
+                   const int64_t* prior_keys, const int64_t* prior_counts, int64_t n_prior, int64_t* digits,
+                   int64_t digit_stride, int64_t* run_keys, int64_t* run_counts, int64_t* stats, void* workspace,
+                   size_t workspace_bytes, void* stream);
+
+/*
  * Gumbel-softmax quantiser level, training mode (modules/quantize.py:108-130,144; distributions/gumbel.py:8-18) -- the
  * [N, K] tables of the reference (dist, noise, logits, weights and their autograd copies) never exist in memory:
  *   dist_k = |x|^2 + |c_k|^2 - 2 x.c_k;  ids = argmin_k dist_k;  g_k = -log(-log(u_k + 1e-20) + 1e-20);
