@@ -218,7 +218,9 @@ int hv_gumbel_backward(const float* x, int64_t n, int d, const float* codebook, 
  * stack of modules/encoder.py:23-36 as called by HRqVae.encode (modules/h_rqvae.py:599) in eval / bulk-assignment passes
  * (modules/tokenizer/h_semids.py:127).  One kernel: the chain of GEMMs runs on tcgen05 with the hidden activations kept
  * in tensor memory.  Operands are rounded to fp16 (TF32-grade significand: the precision of the reference's own GPU path,
- * modules/h_rqvae.py:21), accumulation and activations are fp32.
+ * modules/h_rqvae.py:21) with round to nearest even and saturation to +-65504; fp16 subnormals are kept.  Products
+ * accumulate in fp32 and SiLU is evaluated in fp32; each hidden activation is then rounded to fp16 in the same way, as the
+ * next GEMM's operand.  The output layer and the normalisation stay in fp32.
  *   dims        [n_layers + 1] HOST array: input, hidden..., output widths.  Served: {768, 512, 256, 128, 32}; any other
  *               shape returns HV_ERR_UNSUPPORTED / a zero workspace size (the caller keeps its cuBLAS path).
  *   weights     HOST array of n_layers DEVICE pointers, layer l = nn.Linear.weight [dims[l+1], dims[l]] fp32 row-major
@@ -235,8 +237,10 @@ int hv_encoder_forward(const float* x, int64_t n, int n_layers, const int* dims,
 /*
  * The same pass for items stored in half precision: x_f16 [N, dims[0]] fp16 row-major (a catalogue kept as fp16 moves half
  * the bytes over PCIe and out of HBM; the reference keeps its item embeddings as a float tensor it slices per batch,
- * modules/tokenizer/h_semids.py:120-127).  hv_encoder_forward rounds fp32 items to fp16 (round to nearest even) before the
- * first GEMM, so items that are the rounded fp32 items give bit-identical z.
+ * modules/tokenizer/h_semids.py:120-127).  hv_encoder_forward rounds fp32 items to fp16 (round to nearest even, saturating
+ * to +-65504) before the first GEMM, so items that are the rounded fp32 items give bit-identical z.  That holds for every
+ * item with |x| < 65520, where the fp32-to-fp16 conversion (x.half()) is finite.  From 65520 on, x.half() is inf while
+ * hv_encoder_forward saturates the entry to +-65504; x.clamp(-65504, 65504).half() gives the fp32 entry's z there too.
  */
 int hv_encoder_forward_f16(const void* x_f16, int64_t n, int n_layers, const int* dims, const void* workspace, size_t workspace_bytes,
                            int normalize, int precise_silu, float* z, void* stream);
