@@ -19,7 +19,9 @@
 //   NOISE     `uniforms` [N, K] (the reference's torch.rand draw: parity tests) or, when NULL, counter-based Philox4x32-10:
 //             element (n, k) is output (k >> 5) & 3 of the block with key = seed and counter = offset +
 //             (n * 32 + (k & 31)) * ceil(K / 128) + (k >> 7)  -- the lane that owns the code generates it, four codes per
-//             call, and the backward regenerates exactly the same draw from (seed, offset).
+//             call, and the backward regenerates exactly the same draw from (seed, offset).  (seed, offset) are host scalars
+//             or, for the *_devrng entries, the pair {seed, offset} in device memory: a seed drawn on the device (by a CUDA
+//             graph, afresh at every replay) gives the same draw as the host seed of the same value.
 // Served: D in {16, 32, 64}, K <= 256 (HiD-VAE: D = 32, K = 256); other shapes report HV_ERR_UNSUPPORTED.
 #include <math.h>
 
@@ -44,6 +46,7 @@ struct GumbelArgs {
   float beta;
   const float* uniforms;  // [N, K] or null
   uint64_t seed, offset;
+  const uint64_t* rng;    // device {seed, offset}, or null: then seed and offset above
   // forward outputs / backward inputs
   float* emb_out;   // [N, D]
   int64_t* ids;     // [N] (forward) or null
@@ -76,12 +79,24 @@ __device__ __forceinline__ uint4 philox4x32_10(uint2 key, uint4 c) {
   return c;
 }
 
+// the Philox stream of a call: key = seed, counters from offset
+struct Stream {
+  uint2 key;
+  uint64_t offset;
+};
+
+// read once per thread (the backward: once per CTA, into shared memory), before the row loop
+__device__ __forceinline__ Stream stream_of(const GumbelArgs& a) {
+  uint64_t seed = a.seed, offset = a.offset;
+  if (a.rng != nullptr) seed = a.rng[0], offset = a.rng[1];
+  return {make_uint2(static_cast<uint32_t>(seed), static_cast<uint32_t>(seed >> 32)), offset};
+}
+
 // the uniforms of codes k = lane + 32 j, j in [4 jq, 4 jq + 4), of row n
-__device__ __forceinline__ void draw4(const GumbelArgs& a, int64_t n, int lane, int jq, int blocks_per_lane, float (&u)[4]) {
-  const uint64_t ctr = a.offset + (static_cast<uint64_t>(n) * 32u + static_cast<uint64_t>(lane)) * static_cast<uint64_t>(blocks_per_lane) +
+__device__ __forceinline__ void draw4(const Stream& st, int64_t n, int lane, int jq, int blocks_per_lane, float (&u)[4]) {
+  const uint64_t ctr = st.offset + (static_cast<uint64_t>(n) * 32u + static_cast<uint64_t>(lane)) * static_cast<uint64_t>(blocks_per_lane) +
                        static_cast<uint64_t>(jq);
-  const uint4 r = philox4x32_10(make_uint2(static_cast<uint32_t>(a.seed), static_cast<uint32_t>(a.seed >> 32)),
-                                make_uint4(static_cast<uint32_t>(ctr), static_cast<uint32_t>(ctr >> 32), 0u, 0u));
+  const uint4 r = philox4x32_10(st.key, make_uint4(static_cast<uint32_t>(ctr), static_cast<uint32_t>(ctr >> 32), 0u, 0u));
   constexpr float kScale = 5.9604644775390625e-08f;  // 2^-24: 24-bit uniforms in [0, 1) like torch.rand
   u[0] = static_cast<float>(r.x >> 8) * kScale;
   u[1] = static_cast<float>(r.y >> 8) * kScale;
@@ -173,6 +188,7 @@ __global__ void __launch_bounds__(kThreads) gumbel_fwd_kernel(GumbelArgs a) {
 
   const int warp = ptx::warp_index(), lane = threadIdx.x & 31;
   const int blocks_per_lane = (a.k + 127) / 128;
+  const Stream st = stream_of(a);
   for (int64_t row = static_cast<int64_t>(blockIdx.x) * kWarps + warp; row < a.n; row += static_cast<int64_t>(gridDim.x) * kWarps) {
     float x[D];
     load_row<D>(x, a.x + row * D);
@@ -193,7 +209,7 @@ __global__ void __launch_bounds__(kThreads) gumbel_fwd_kernel(GumbelArgs a) {
       if (a.uniforms != nullptr) {
         u = __ldg(a.uniforms + row * a.k + k);
       } else {
-        if ((j & 3) == 0) draw4(a, row, lane, j >> 2, blocks_per_lane, u4);
+        if ((j & 3) == 0) draw4(st, row, lane, j >> 2, blocks_per_lane, u4);
         u = u4[j & 3];
       }
       const float y = __fdiv_rn(gumbel_of(u) - dist, a.temperature);  // (logits + G) / T, logits = -dist
@@ -252,10 +268,14 @@ __global__ void __launch_bounds__(kThreads) gumbel_bwd_kernel(GumbelArgs a) {
   float* s_x = s_a + kTile * kMaxK;                     // [kTile][D]
   float* s_ge = s_x + kTile * D;                        // [kTile][D]
   float* s_red = s_ge + kTile * D + (threadIdx.x >> 5) * 32 * (D + 1);
+  // the stream stays in shared memory: at D = 64 the row loop already spills, and four more live registers would add spills
+  __shared__ Stream s_st;
+  if (threadIdx.x == 0) s_st = stream_of(a);  // (made visible by load_codebook's barrier)
   load_codebook<D>(a, s_cb, s_cn);
 
   const int warp = ptx::warp_index(), lane = threadIdx.x & 31;
   const int blocks_per_lane = (a.k + 127) / 128;
+  const Stream& st = s_st;
   const float inv_t = 1.0f / a.temperature;
   float acc[D];
 #pragma unroll
@@ -307,7 +327,7 @@ __global__ void __launch_bounds__(kThreads) gumbel_bwd_kernel(GumbelArgs a) {
         if (a.uniforms != nullptr) {
           u = __ldg(a.uniforms + row * a.k + k);
         } else {
-          if ((j & 3) == 0) draw4(a, row, lane, j >> 2, blocks_per_lane, u4);
+          if ((j & 3) == 0) draw4(st, row, lane, j >> 2, blocks_per_lane, u4);
           u = u4[j & 3];
         }
         const float y = __fdiv_rn(gumbel_of(u) - dist, a.temperature);
@@ -365,12 +385,13 @@ __global__ void __launch_bounds__(kThreads) gumbel_bwd_kernel(GumbelArgs a) {
 __global__ void __launch_bounds__(kThreads) gumbel_uniforms_kernel(GumbelArgs a, float* __restrict__ out) {
   const int blocks_per_lane = (a.k + 127) / 128;
   const int64_t total = a.n * 32 * blocks_per_lane;  // one Philox block per thread
+  const Stream st = stream_of(a);
   for (int64_t i = static_cast<int64_t>(blockIdx.x) * kThreads + threadIdx.x; i < total; i += static_cast<int64_t>(gridDim.x) * kThreads) {
     const int jq = static_cast<int>(i % blocks_per_lane);
     const int lane = static_cast<int>((i / blocks_per_lane) % 32);
     const int64_t row = i / (static_cast<int64_t>(blocks_per_lane) * 32);
     float u4[4];
-    draw4(a, row, lane, jq, blocks_per_lane, u4);
+    draw4(st, row, lane, jq, blocks_per_lane, u4);
 #pragma unroll
     for (int t = 0; t < 4; ++t) {
       const int k = lane + 32 * (4 * jq + t);
@@ -428,24 +449,20 @@ int check_common(const char* who, const float* x, int64_t n, int d, const float*
   return HV_OK;
 }
 
-}  // namespace
-}  // namespace hv
-
-extern "C" int hv_gumbel_supported(int d, int k) { return (d == 16 || d == 32 || d == 64) && k >= 1 && k <= hv::kMaxK; }
-
-extern "C" int hv_gumbel_uniforms(int64_t n, int k, uint64_t seed, uint64_t offset, float* uniforms, void* stream) {
-  using namespace hv;
+// The host-seed entries pass (seed, offset) and rng = null; the *_devrng entries pass rng, which must be non-null when n > 0.
+int uniforms_impl(const char* who, int64_t n, int k, uint64_t seed, uint64_t offset, const uint64_t* rng, bool devrng,
+                  float* uniforms, void* stream) {
   if (n < 0 || k <= 0) {
-    set_error("hv_gumbel_uniforms: bad shape n=%lld k=%d", static_cast<long long>(n), k);
+    set_error("%s: bad shape n=%lld k=%d", who, static_cast<long long>(n), k);
     return HV_ERR_BAD_SHAPE;
   }
   if (n == 0) return HV_OK;
-  if (!uniforms) {
-    set_error("hv_gumbel_uniforms: null pointer");
+  if (!uniforms || (devrng && !rng)) {
+    set_error("%s: null pointer", who);
     return HV_ERR_NULL;
   }
   GumbelArgs a{};
-  a.n = n, a.k = k, a.seed = seed, a.offset = offset;
+  a.n = n, a.k = k, a.seed = seed, a.offset = offset, a.rng = rng;
   const int64_t total = n * 32 * ((k + 127) / 128);
   const int64_t blocks = (total + kThreads - 1) / kThreads;
   gumbel_uniforms_kernel<<<static_cast<unsigned>(blocks < 65535 ? blocks : 65535), kThreads, 0, static_cast<cudaStream_t>(stream)>>>(a, uniforms);
@@ -453,21 +470,24 @@ extern "C" int hv_gumbel_uniforms(int64_t n, int k, uint64_t seed, uint64_t offs
   return HV_OK;
 }
 
-extern "C" int hv_gumbel_forward(const float* x, int64_t n, int d, const float* codebook, int k, float temperature, float beta,
-                                 const float* uniforms, uint64_t seed, uint64_t offset, float* emb_out, int64_t* ids, float* loss,
-                                 float* lse, void* stream) {
-  using namespace hv;
-  if (int st = check_common("hv_gumbel_forward", x, n, d, codebook, k, temperature)) return st;
+int forward_impl(const char* who, const float* x, int64_t n, int d, const float* codebook, int k, float temperature, float beta,
+                 const float* uniforms, uint64_t seed, uint64_t offset, const uint64_t* rng, bool devrng, float* emb_out,
+                 int64_t* ids, float* loss, float* lse, void* stream) {
+  if (int st = check_common(who, x, n, d, codebook, k, temperature)) return st;
   if (n == 0) return HV_OK;
   if (!emb_out || !lse) {
-    set_error("hv_gumbel_forward: emb_out and lse are required");
+    set_error("%s: emb_out and lse are required", who);
+    return HV_ERR_NULL;
+  }
+  if (devrng && !rng) {
+    set_error("%s: rng (the device pair {seed, offset}) is required", who);
     return HV_ERR_NULL;
   }
   DeviceProps props;
   if (int st = device_props(&props)) return st;
   GumbelArgs a{};
   a.x = x, a.codebook = codebook, a.n = n, a.k = k, a.temperature = temperature, a.beta = beta;
-  a.uniforms = uniforms, a.seed = seed, a.offset = offset;
+  a.uniforms = uniforms, a.seed = seed, a.offset = offset, a.rng = rng;
   a.emb_out = emb_out, a.ids = ids, a.loss = loss, a.lse = lse;
   cudaStream_t s = static_cast<cudaStream_t>(stream);
   switch (d) {
@@ -477,25 +497,28 @@ extern "C" int hv_gumbel_forward(const float* x, int64_t n, int d, const float* 
   }
 }
 
-extern "C" int hv_gumbel_backward(const float* x, int64_t n, int d, const float* codebook, int k, float temperature, float beta,
-                                  const float* uniforms, uint64_t seed, uint64_t offset, const float* emb_out, const float* lse,
-                                  const float* g_emb, const float* g_loss, float* g_x, float* g_codebook, void* stream) {
-  using namespace hv;
-  if (int st = check_common("hv_gumbel_backward", x, n, d, codebook, k, temperature)) return st;
+int backward_impl(const char* who, const float* x, int64_t n, int d, const float* codebook, int k, float temperature, float beta,
+                  const float* uniforms, uint64_t seed, uint64_t offset, const uint64_t* rng, bool devrng, const float* emb_out,
+                  const float* lse, const float* g_emb, const float* g_loss, float* g_x, float* g_codebook, void* stream) {
+  if (int st = check_common(who, x, n, d, codebook, k, temperature)) return st;
   if (n == 0) return HV_OK;
   if (!emb_out || !lse || !g_x || !g_codebook) {
-    set_error("hv_gumbel_backward: emb_out, lse, g_x and g_codebook are required");
+    set_error("%s: emb_out, lse, g_x and g_codebook are required", who);
+    return HV_ERR_NULL;
+  }
+  if (devrng && !rng) {
+    set_error("%s: rng (the device pair {seed, offset}) is required", who);
     return HV_ERR_NULL;
   }
   if (!aligned16(emb_out) || !aligned16(g_emb)) {
-    set_error("hv_gumbel_backward: emb_out and g_emb must be 16-byte aligned");
+    set_error("%s: emb_out and g_emb must be 16-byte aligned", who);
     return HV_ERR_MISALIGNED;
   }
   DeviceProps props;
   if (int st = device_props(&props)) return st;
   GumbelArgs a{};
   a.x = x, a.codebook = codebook, a.n = n, a.k = k, a.temperature = temperature, a.beta = beta;
-  a.uniforms = uniforms, a.seed = seed, a.offset = offset;
+  a.uniforms = uniforms, a.seed = seed, a.offset = offset, a.rng = rng;
   a.emb_out = const_cast<float*>(emb_out), a.lse = const_cast<float*>(lse);
   a.g_emb = g_emb, a.g_loss = g_loss, a.g_x = g_x, a.g_codebook = g_codebook;
   cudaStream_t s = static_cast<cudaStream_t>(stream);
@@ -504,4 +527,46 @@ extern "C" int hv_gumbel_backward(const float* x, int64_t n, int d, const float*
     case 32: return launch_bwd<32>(a, props.sm_count, s);
     default: return launch_bwd<64>(a, props.sm_count, s);
   }
+}
+
+}  // namespace
+}  // namespace hv
+
+extern "C" int hv_gumbel_supported(int d, int k) { return (d == 16 || d == 32 || d == 64) && k >= 1 && k <= hv::kMaxK; }
+
+extern "C" int hv_gumbel_uniforms(int64_t n, int k, uint64_t seed, uint64_t offset, float* uniforms, void* stream) {
+  return hv::uniforms_impl("hv_gumbel_uniforms", n, k, seed, offset, nullptr, false, uniforms, stream);
+}
+
+extern "C" int hv_gumbel_uniforms_devrng(int64_t n, int k, const uint64_t* rng, float* uniforms, void* stream) {
+  return hv::uniforms_impl("hv_gumbel_uniforms_devrng", n, k, 0, 0, rng, true, uniforms, stream);
+}
+
+extern "C" int hv_gumbel_forward(const float* x, int64_t n, int d, const float* codebook, int k, float temperature, float beta,
+                                 const float* uniforms, uint64_t seed, uint64_t offset, float* emb_out, int64_t* ids, float* loss,
+                                 float* lse, void* stream) {
+  return hv::forward_impl("hv_gumbel_forward", x, n, d, codebook, k, temperature, beta, uniforms, seed, offset, nullptr, false,
+                          emb_out, ids, loss, lse, stream);
+}
+
+extern "C" int hv_gumbel_forward_devrng(const float* x, int64_t n, int d, const float* codebook, int k, float temperature,
+                                        float beta, const float* uniforms, const uint64_t* rng, float* emb_out, int64_t* ids,
+                                        float* loss, float* lse, void* stream) {
+  return hv::forward_impl("hv_gumbel_forward_devrng", x, n, d, codebook, k, temperature, beta, uniforms, 0, 0, rng, true,
+                          emb_out, ids, loss, lse, stream);
+}
+
+extern "C" int hv_gumbel_backward(const float* x, int64_t n, int d, const float* codebook, int k, float temperature, float beta,
+                                  const float* uniforms, uint64_t seed, uint64_t offset, const float* emb_out, const float* lse,
+                                  const float* g_emb, const float* g_loss, float* g_x, float* g_codebook, void* stream) {
+  return hv::backward_impl("hv_gumbel_backward", x, n, d, codebook, k, temperature, beta, uniforms, seed, offset, nullptr, false,
+                           emb_out, lse, g_emb, g_loss, g_x, g_codebook, stream);
+}
+
+extern "C" int hv_gumbel_backward_devrng(const float* x, int64_t n, int d, const float* codebook, int k, float temperature,
+                                         float beta, const float* uniforms, const uint64_t* rng, const float* emb_out,
+                                         const float* lse, const float* g_emb, const float* g_loss, float* g_x,
+                                         float* g_codebook, void* stream) {
+  return hv::backward_impl("hv_gumbel_backward_devrng", x, n, d, codebook, k, temperature, beta, uniforms, 0, 0, rng, true,
+                           emb_out, lse, g_emb, g_loss, g_x, g_codebook, stream);
 }

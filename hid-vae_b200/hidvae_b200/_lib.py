@@ -58,6 +58,11 @@ SIGNATURES = {
                                   c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "hv_gumbel_backward": (c_int, [c_void_p, c_int64, c_int, c_void_p, c_int, c_float, c_float, c_void_p, c_uint64, c_uint64,
                                    c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "hv_gumbel_uniforms_devrng": (c_int, [c_int64, c_int, c_void_p, c_void_p, c_void_p]),
+    "hv_gumbel_forward_devrng": (c_int, [c_void_p, c_int64, c_int, c_void_p, c_int, c_float, c_float, c_void_p, c_void_p,
+                                         c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
+    "hv_gumbel_backward_devrng": (c_int, [c_void_p, c_int64, c_int, c_void_p, c_int, c_float, c_float, c_void_p, c_void_p,
+                                          c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p]),
     "hv_encoder_workspace_bytes": (c_size_t, [c_int, POINTER(c_int)]),
     "hv_encoder_pack_weights": (c_int, [POINTER(c_void_p), c_int, POINTER(c_int), c_void_p, c_size_t, c_void_p]),
     "hv_encoder_forward": (c_int, [c_void_p, c_int64, c_int, POINTER(c_int), c_void_p, c_size_t, c_int, c_int, c_void_p,

@@ -13,9 +13,11 @@ once, after a few eager warm-up steps on the capture stream, and replays them.  
 exchange runs eagerly: one NCCL all-reduce of the flat buffer (`FlatGradAllReduce.all_reduce`); with one process the two
 replays are back to back.  Requirements, checked at construction: no fp16 loss scaling (its inf check reads back to the
 host), a model whose forward is free of host synchronisation (HRqVae is: the tag losses are masked fixed-shape means, the
-uniqueness loss and p_unique_ids are kernels), fixed batch size, STE / rotation-trick quantiser (the Gumbel-softmax kernels
-take their noise seed as a host scalar, which a graph would freeze: `ops.gumbel_apply` refuses to be captured).  Dropout and
-mixup draws advance inside the graph through PyTorch's graph-safe Philox offsets.  No autograd graph of an EARLIER eager
+uniqueness loss and p_unique_ids are kernels), fixed batch size.  Dropout and mixup draws advance inside the graph through
+PyTorch's graph-safe Philox offsets, and so do the Gumbel-softmax levels: under capture `ops.gumbel_apply` draws each level's
+noise seed on the device, so every replay draws new noise, and the forward and backward of one replay read the same seed.
+`gumbel_t` is a host scalar and is frozen at capture; the trainer's temperature is the constant 0.2 of the reference, so
+nothing is lost there, but a temperature schedule would need a new capture per value.  No autograd graph of an EARLIER eager
 step may still be alive when this is built (e.g. a kept `out.loss`): its AccumulateGrad nodes are bound to the stream they
 ran on, and the capture would have to synchronise with it.  The warm-up steps are REAL optimisation
 steps (with the gradient exchange): a run with `warmup` = 3 has made three steps when the constructor returns."""

@@ -212,25 +212,52 @@ def gumbel_supported(d: int, k: int) -> bool:
     return bool(lib.hv_gumbel_supported(int(d), int(k)))
 
 
-def gumbel_uniforms(n: int, k: int, seed: int, device) -> Tensor:
-    """The [N, K] uniforms the fused Gumbel kernels draw for `seed` (recording / reproducing a step)."""
-    out = torch.empty((n, k), dtype=torch.float32, device=device)
+def _device_rng(seed, device=None) -> Optional[Tensor]:
+    """None for a host seed (a Python int); for a device seed the validated tensor (seed, offset): a CUDA int64 of two
+    elements with values in [0, 2^62), on `device` when one is given."""
+    if not isinstance(seed, Tensor):
+        return None
+    if not seed.is_cuda or seed.dtype != torch.int64 or seed.numel() != 2:
+        raise ValueError("a device Gumbel seed is a CUDA int64 tensor of two elements (seed, offset); got "
+                         f"{seed.dtype} {tuple(seed.shape)} on {seed.device}")
+    if device is not None:
+        device = torch.device(device)
+        if device.type == "cuda" and device.index is None:
+            device = torch.device("cuda", torch.cuda.current_device())
+        if seed.device != device:
+            raise ValueError(f"the device Gumbel seed is on {seed.device}, the operands on {device}")
+    return seed.reshape(2).contiguous()
+
+
+def gumbel_uniforms(n: int, k: int, seed, device=None) -> Tensor:
+    """The [N, K] uniforms the fused Gumbel kernels draw for `seed` (recording / reproducing a step): a Python int, or a
+    device pair (seed, offset) such as the one `gumbel_apply` saved (`device` then defaults to the pair's)."""
+    rng = _device_rng(seed, device)
+    out = torch.empty((n, k), dtype=torch.float32, device=device if rng is None else rng.device)
     with torch.cuda.device(out.device):
-        check(lib.hv_gumbel_uniforms(n, k, int(seed), 0, out.data_ptr(), _stream(out)))
+        if rng is None:
+            check(lib.hv_gumbel_uniforms(n, k, int(seed), 0, out.data_ptr(), _stream(out)))
+        else:
+            check(lib.hv_gumbel_uniforms_devrng(n, k, rng.data_ptr(), out.data_ptr(), _stream(out)))
     return out
 
 
 class GumbelFunction(torch.autograd.Function):
     """Fused Gumbel-softmax level: forward(x [N, D], codebook [K, D], temperature, beta, uniforms [N, K] | None, seed)
     -> emb_out [N, D], ids [N] (not differentiable), loss [N].  The noise is either the given uniforms (the reference's
-    torch.rand draw) or Philox uniforms of `seed`, regenerated in the backward; dist / logits / weights never reach HBM."""
+    torch.rand draw) or Philox uniforms of `seed`, regenerated in the backward; dist / logits / weights never reach HBM.
+    `seed` is a Python int or a CUDA int64 tensor (seed, offset) read by the kernels on the device; the backward reads the
+    tensor the forward saved (the last of ctx.saved_tensors)."""
 
     @staticmethod
     def forward(ctx, x, codebook, temperature, beta, uniforms, seed):
+        rng = _device_rng(seed)
         _require_cuda(x, codebook)
         x, codebook = _f32c(x), _f32c(codebook)
         n, d = x.shape
         k = codebook.shape[0]
+        if rng is not None and rng.device != x.device:
+            raise ValueError(f"the device Gumbel seed is on {rng.device}, x on {x.device}")
         if uniforms is not None:
             _require_cuda(uniforms)
             uniforms = _f32c(uniforms)
@@ -240,17 +267,22 @@ class GumbelFunction(torch.autograd.Function):
         loss = torch.empty((n,), dtype=torch.float32, device=x.device)
         lse = torch.empty((n,), dtype=torch.float32, device=x.device)
         with torch.cuda.device(x.device):
-            check(lib.hv_gumbel_forward(x.data_ptr(), n, d, codebook.data_ptr(), k, float(temperature), float(beta), _ptr(uniforms),
-                                        int(seed), 0, emb.data_ptr(), ids.data_ptr(), loss.data_ptr(), lse.data_ptr(), _stream(x)))
-        ctx.save_for_backward(x, codebook, emb, lse, *([uniforms] if uniforms is not None else []))
-        ctx.cfg = (float(temperature), float(beta), int(seed))
+            if rng is None:
+                check(lib.hv_gumbel_forward(x.data_ptr(), n, d, codebook.data_ptr(), k, float(temperature), float(beta),
+                                            _ptr(uniforms), int(seed), 0, emb.data_ptr(), ids.data_ptr(), loss.data_ptr(),
+                                            lse.data_ptr(), _stream(x)))
+            else:
+                check(lib.hv_gumbel_forward_devrng(x.data_ptr(), n, d, codebook.data_ptr(), k, float(temperature), float(beta),
+                                                   _ptr(uniforms), rng.data_ptr(), emb.data_ptr(), ids.data_ptr(),
+                                                   loss.data_ptr(), lse.data_ptr(), _stream(x)))
+        ctx.save_for_backward(x, codebook, emb, lse, uniforms, rng)
+        ctx.cfg = (float(temperature), float(beta), None if rng is not None else int(seed))
         ctx.mark_non_differentiable(ids)
         return emb, ids, loss
 
     @staticmethod
     def backward(ctx, g_emb, _g_ids, g_loss):
-        x, codebook, emb, lse, *rest = ctx.saved_tensors
-        uniforms = rest[0] if rest else None
+        x, codebook, emb, lse, uniforms, rng = ctx.saved_tensors
         temperature, beta, seed = ctx.cfg
         n, d = x.shape
         k = codebook.shape[0]
@@ -259,22 +291,34 @@ class GumbelFunction(torch.autograd.Function):
         g_x = torch.empty_like(x)
         g_cb = torch.zeros_like(codebook)
         with torch.cuda.device(x.device):
-            check(lib.hv_gumbel_backward(x.data_ptr(), n, d, codebook.data_ptr(), k, temperature, beta, _ptr(uniforms), seed, 0,
-                                         emb.data_ptr(), lse.data_ptr(), _ptr(g_emb), _ptr(g_loss), g_x.data_ptr(), g_cb.data_ptr(),
-                                         _stream(x)))
+            if rng is None:
+                check(lib.hv_gumbel_backward(x.data_ptr(), n, d, codebook.data_ptr(), k, temperature, beta, _ptr(uniforms), seed,
+                                             0, emb.data_ptr(), lse.data_ptr(), _ptr(g_emb), _ptr(g_loss), g_x.data_ptr(),
+                                             g_cb.data_ptr(), _stream(x)))
+            else:
+                check(lib.hv_gumbel_backward_devrng(x.data_ptr(), n, d, codebook.data_ptr(), k, temperature, beta,
+                                                    _ptr(uniforms), rng.data_ptr(), emb.data_ptr(), lse.data_ptr(), _ptr(g_emb),
+                                                    _ptr(g_loss), g_x.data_ptr(), g_cb.data_ptr(), _stream(x)))
         return g_x, g_cb, None, None, None, None
 
 
 def gumbel_apply(x: Tensor, codebook: Tensor, temperature: float, beta: float, uniforms: Optional[Tensor] = None,
-                 seed: Optional[int] = None):
+                 seed=None):
     """(emb_out [N, D], ids [N], loss [N]) of one Gumbel-softmax level.  Without `uniforms` the noise comes from Philox with
-    `seed` (default: a fresh draw from torch's CPU generator, so torch.manual_seed makes a run reproducible)."""
+    `seed`: a Python int, or a CUDA int64 tensor (seed, offset) read on the device.  The default draws a fresh seed: eagerly
+    from torch's CPU generator (so torch.manual_seed makes a run reproducible); under CUDA-graph capture as a (seed, 0)
+    tensor from torch's CUDA generator, so that every replay of the graph draws anew."""
     if seed is None:
         if torch.cuda.is_current_stream_capturing():
-            raise RuntimeError("gumbel_apply under CUDA-graph capture: the noise seed is a host scalar and would be frozen into "
-                               "the graph (every replay the same draw); run Gumbel-softmax steps eagerly")
-        seed = int(torch.randint(0, 2 ** 62, (1,)).item())
-    return GumbelFunction.apply(x, codebook, float(temperature), float(beta), uniforms, int(seed))
+            # a host draw would be frozen into the graph; torch's CUDA generator is graph-safe: every replay advances its
+            # Philox offset, so every replay draws a new seed
+            seed = torch.zeros(2, dtype=torch.int64, device=x.device)
+            seed[:1].random_(0, 2 ** 62)
+        else:
+            seed = int(torch.randint(0, 2 ** 62, (1,)).item())
+    elif not isinstance(seed, Tensor):
+        seed = int(seed)
+    return GumbelFunction.apply(x, codebook, float(temperature), float(beta), uniforms, seed)
 
 
 def _dims_array(dims):

@@ -144,7 +144,7 @@ def train(
     seed=0,
     uniqueness_as_reference=True,
     use_cuda_graph=False,      # replay the micro-step (gather + forward + backward) and the AdamW step as CUDA graphs
-                               # (hidvae_b200/graph_step.py); not with fp16 loss scaling or the Gumbel-softmax mode
+                               # (hidvae_b200/graph_step.py); not with fp16 loss scaling
 ):
     rank, world, local = hv_dist.init_from_env()
     is_main = rank == 0
@@ -225,8 +225,6 @@ def train(
         if use_cuda_graph:
             if bool(amp) and mixed_precision_type == "fp16":
                 raise ValueError("train.use_cuda_graph: fp16 loss scaling reads its inf check back to the host; use bf16 or amp=False")
-            if vae_codebook_mode == QuantizeForwardMode.GUMBEL_SOFTMAX:
-                raise ValueError("train.use_cuda_graph: the Gumbel-softmax noise seed is a host scalar; use STE or ROTATION_TRICK")
             for g_ in optimizer.param_groups:      # the graph reads the learning rate from device memory: the scheduler updates it in place
                 g_["lr"] = torch.tensor(float(g_["lr"]), device=device)
 

@@ -203,6 +203,11 @@ int hv_semid_dedup(const int64_t* ids, int64_t rows, int64_t width, int64_t row_
  * Served shapes: D in {16, 32, 64}, K <= 256 (hv_gumbel_supported); others return HV_ERR_UNSUPPORTED.
  * hv_gumbel_uniforms writes the [N, K] uniforms the two kernels generate for (seed, offset): recording a step's draw, and
  *   the test that the Philox path equals the explicit-noise path.
+ * The *_devrng entries are their counterparts with the pair in device memory: rng points at two uint64 {seed, offset},
+ *   read by the kernels when they run, so a CUDA graph can draw a fresh seed on the device before every replay (the forward
+ *   and backward of one replay read the same pair).  A pair gives the same draw as the host scalars of the same values.
+ *   Argument errors return before any CUDA call (a NULL rng with n > 0: HV_ERR_NULL); n = 0 is a no-op; like the host-seed
+ *   entries they allocate nothing and do not synchronise with the host.
  */
 int hv_gumbel_supported(int d, int k);
 int hv_gumbel_uniforms(int64_t n, int k, uint64_t seed, uint64_t offset, float* uniforms, void* stream);
@@ -212,6 +217,13 @@ int hv_gumbel_forward(const float* x, int64_t n, int d, const float* codebook, i
 int hv_gumbel_backward(const float* x, int64_t n, int d, const float* codebook, int k, float temperature, float beta,
                        const float* uniforms, uint64_t seed, uint64_t offset, const float* emb_out, const float* lse,
                        const float* g_emb, const float* g_loss, float* g_x, float* g_codebook, void* stream);
+int hv_gumbel_uniforms_devrng(int64_t n, int k, const uint64_t* rng, float* uniforms, void* stream);
+int hv_gumbel_forward_devrng(const float* x, int64_t n, int d, const float* codebook, int k, float temperature, float beta,
+                             const float* uniforms, const uint64_t* rng, float* emb_out, int64_t* ids, float* loss, float* lse,
+                             void* stream);
+int hv_gumbel_backward_devrng(const float* x, int64_t n, int d, const float* codebook, int k, float temperature, float beta,
+                              const float* uniforms, const uint64_t* rng, const float* emb_out, const float* lse,
+                              const float* g_emb, const float* g_loss, float* g_x, float* g_codebook, void* stream);
 
 /*
  * Fused encoder MLP in front of the quantiser: z = [l2norm](W_L silu(... silu(W_1 x))) -- the bias-free Linear + SiLU
