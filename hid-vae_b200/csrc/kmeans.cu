@@ -5,7 +5,10 @@
 //   hv_kmeans_accumulate  per-cluster sums / counts of the assigned rows, bit-reproducible from run to run.  That
 //                         matters: the reference stops when max ||c_new - c_old|| < 1e-10 (init/kmeans.py:68), i.e.
 //                         when the update reproduces the centroids exactly, which an atomics-ordered float sum never does.
-//                         Two forms, chosen by shape only:
+//                         Every row chain is a compensated (Kahan) sum in a fixed order: its error stays about two
+//                         ulps of sum |x| however many rows a cluster holds (a plain fp32 chain grows with the chain, to
+//                         1e-2 relative for 2^20 identical rows), and the order keeps the result bit-reproducible.
+//                         Assignments must lie in [0, K).  Two forms, chosen by shape only:
 //                           segmented (needs the sort workspace; O(N)): rows are key-sorted by cluster (stable radix
 //                             sort, sort.cuh) and ONE WARP PER CLUSTER adds its members in row order -- x is read once,
 //                             whatever K is;
@@ -21,6 +24,15 @@ namespace {
 
 constexpr int kAccThreads = 256;
 
+// one step of a compensated sum: s - comp is the running total to about twice fp32's precision (comp holds the
+// negated low part the last addition lost)
+__device__ __forceinline__ void kahan_add(float& s, float& comp, float v) {
+  const float y = v - comp;
+  const float t = s + y;
+  comp = (t - s) - y;
+  s = t;
+}
+
 template <int D>
 __global__ void __launch_bounds__(kAccThreads) kmeans_accumulate_kernel(const float* __restrict__ x, int64_t n,
                                                                         const int64_t* __restrict__ assign,
@@ -32,25 +44,35 @@ __global__ void __launch_bounds__(kAccThreads) kmeans_accumulate_kernel(const fl
   const int tid = threadIdx.x;
   const int lane = tid & 31, warp = ptx::warp_index();
 
-  float acc[D];
+  // thread t adds rows t, t + 256, ... of its cluster in one compensated chain per dimension; the assignments of 4 of its
+  // rows are loaded ahead (independent loads), then the rows are taken in order
+  float acc[D], cmp[D];
 #pragma unroll
-  for (int i = 0; i < D; ++i) acc[i] = 0.f;
+  for (int i = 0; i < D; ++i) acc[i] = 0.f, cmp[i] = 0.f;
   float cnt = 0.f;
-  for (int64_t row = tid; row < n; row += kAccThreads) {
-    if (assign[row] == c) {
-      const float4* src = reinterpret_cast<const float4*>(x + row * D);
+  for (int64_t base = tid; base < n; base += 4 * kAccThreads) {
+    int64_t a4[4];
+#pragma unroll
+    for (int u = 0; u < 4; ++u) a4[u] = base + u * kAccThreads < n ? __ldg(assign + base + u * kAccThreads) : -1;
+#pragma unroll
+    for (int u = 0; u < 4; ++u) {
+      if (a4[u] != c) continue;
+      const float4* src = reinterpret_cast<const float4*>(x + (base + u * kAccThreads) * D);
 #pragma unroll
       for (int i = 0; i < D / 4; ++i) {
         const float4 v = __ldg(src + i);
-        acc[4 * i] += v.x, acc[4 * i + 1] += v.y, acc[4 * i + 2] += v.z, acc[4 * i + 3] += v.w;
+        kahan_add(acc[4 * i], cmp[4 * i], v.x);
+        kahan_add(acc[4 * i + 1], cmp[4 * i + 1], v.y);
+        kahan_add(acc[4 * i + 2], cmp[4 * i + 2], v.z);
+        kahan_add(acc[4 * i + 3], cmp[4 * i + 3], v.w);
       }
       cnt += 1.f;
     }
   }
-  // fixed-shape reduction: xor tree inside the warp, then the 8 warp partials in warp order
+  // fixed-shape reduction of the corrected chains: xor tree inside the warp, then the 8 warp partials in warp order
 #pragma unroll
   for (int i = 0; i < D; ++i) {
-    float v = acc[i];
+    float v = acc[i] - cmp[i];
 #pragma unroll
     for (int off = 16; off > 0; off >>= 1) v += __shfl_xor_sync(0xffffffffu, v, off);
     if (lane == 0) s_part[warp][i] = v;
@@ -113,7 +135,7 @@ __device__ __forceinline__ int64_t lower_bound_u64(const uint64_t* __restrict__ 
 
 // one warp per cluster: its members sit in [lo, hi) of the sorted order, in ascending row order (stable sort); lane l owns
 // dimensions l, l + 32, ...; 32 row indices are fetched per step and their rows are loaded back to back (independent
-// loads), then added in row order -- a fixed summation order whatever the launch shape.
+// loads), then added in row order to one compensated chain per dimension -- a fixed order whatever the launch shape.
 template <int D>
 __global__ void __launch_bounds__(256) kmeans_segsum_kernel(const float* __restrict__ x, int64_t n, const uint64_t* __restrict__ keys,
                                                             const uint32_t* __restrict__ rows, int k, float* __restrict__ sums,
@@ -124,9 +146,9 @@ __global__ void __launch_bounds__(256) kmeans_segsum_kernel(const float* __restr
   if (c >= k) return;
   const int64_t lo = lower_bound_u64(keys, n, static_cast<uint64_t>(c));
   const int64_t hi = lower_bound_u64(keys, n, static_cast<uint64_t>(c) + 1);
-  float acc[PER];
+  float acc[PER], cmp[PER];
 #pragma unroll
-  for (int p = 0; p < PER; ++p) acc[p] = 0.f;
+  for (int p = 0; p < PER; ++p) acc[p] = 0.f, cmp[p] = 0.f;
   for (int64_t base = lo; base < hi; base += 32) {
     const int m = static_cast<int>(hi - base < 32 ? hi - base : 32);
     const uint32_t mine = lane < m ? rows[base + lane] : 0u;
@@ -141,13 +163,14 @@ __global__ void __launch_bounds__(256) kmeans_segsum_kernel(const float* __restr
       }
 #pragma unroll
       for (int t = 0; t < 8; ++t)
+        if (t0 + t < m)
 #pragma unroll
-        for (int p = 0; p < PER; ++p) acc[p] += v[t][p];
+          for (int p = 0; p < PER; ++p) kahan_add(acc[p], cmp[p], v[t][p]);
     }
   }
 #pragma unroll
   for (int p = 0; p < PER; ++p)
-    if (lane + 32 * p < D) sums[static_cast<int64_t>(c) * D + lane + 32 * p] = acc[p];
+    if (lane + 32 * p < D) sums[static_cast<int64_t>(c) * D + lane + 32 * p] = acc[p] - cmp[p];
   if (lane == 0) counts[c] = static_cast<float>(hi - lo);
 }
 

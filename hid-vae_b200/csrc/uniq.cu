@@ -44,7 +44,12 @@ __device__ __forceinline__ bool same_tuple(const UniqArgs& a, int64_t i, int64_t
 }
 
 // cos(f_i, f_j) with F.normalize's eps = 1e-12 clamp on each norm (modules/h_rqvae.py:88-92)
-__device__ __forceinline__ float pair_cos(const UniqArgs& a, int64_t i, int64_t j, float* inv_i, float* inv_j) {
+struct PairCos {
+  float cs, inv_i, inv_j;
+  bool clamped_i, clamped_j;  // the norm is below the clamp: the row is divided by the constant 1e-12
+};
+
+__device__ __forceinline__ PairCos pair_cos(const UniqArgs& a, int64_t i, int64_t j) {
   const float* fi = a.feats + i * a.d;
   const float* fj = a.feats + j * a.d;
   float ii = 0.f, jj = 0.f, ij = 0.f;
@@ -52,9 +57,59 @@ __device__ __forceinline__ float pair_cos(const UniqArgs& a, int64_t i, int64_t 
     const float u = fi[c], v = fj[c];
     ii = fmaf(u, u, ii), jj = fmaf(v, v, jj), ij = fmaf(u, v, ij);
   }
-  *inv_i = 1.0f / fmaxf(sqrtf(ii), 1e-12f);
-  *inv_j = 1.0f / fmaxf(sqrtf(jj), 1e-12f);
-  return ij * (*inv_i) * (*inv_j);
+  PairCos p;
+  const float ni = sqrtf(ii), nj = sqrtf(jj);
+  p.clamped_i = ni < 1e-12f, p.clamped_j = nj < 1e-12f;
+  p.inv_i = 1.0f / fmaxf(ni, 1e-12f);
+  p.inv_j = 1.0f / fmaxf(nj, 1e-12f);
+  p.cs = ij * p.inv_i * p.inv_j;
+  return p;
+}
+
+// g_feats[i] += coef * d cos / d f_i and g_feats[j] += coef * d cos / d f_j.
+// Above the clamp, d cos / d f_i = P_i e / |f_i| with e = fhat_j - fhat_i and P_i = I - fhat_i fhat_i^T (P_i fhat_i = 0):
+// the same vector as (fhat_j - cos fhat_i) / |f_i|, without its cancellation.  With s the row of the smaller norm and
+// inv_lo the other row's inverse norm, e = (f_j - f_i) inv_lo + f_s (inv_j - inv_i): no term exceeds 2 in size, f_j - f_i
+// is exact for near-identical rows, and the rounding of the two norms only moves e along f_s, which P_s removes (and the
+// other row's P up to |e|).  So near-identical rows keep fp32's relative precision, and identical rows get exactly 0 (the
+// products are kept out of FMA contraction for that).  Below the clamp, the row is divided by the constant 1e-12, whose
+// derivative is zero: d cos / d f_i = fhat_j * inv_i, no projection.
+__device__ __forceinline__ void pair_grad(const UniqArgs& a, int64_t i, int64_t j, const PairCos& p, float coef,
+                                          float* __restrict__ g_feats) {
+  const float* fi = a.feats + i * a.d;
+  const float* fj = a.feats + j * a.d;
+  const bool j_small = p.inv_j >= p.inv_i;
+  const float* fs = j_small ? fj : fi;
+  const float inv_lo = j_small ? p.inv_i : p.inv_j;
+  const float dinv = p.inv_j - p.inv_i;
+  float si = 0.f, sj = 0.f;  // fhat_i . e, fhat_j . e
+  for (int c = 0; c < a.d; ++c) {
+    const float e = fmaf(fj[c] - fi[c], inv_lo, __fmul_rn(fs[c], dinv));
+    si = fmaf(__fmul_rn(fi[c], p.inv_i), e, si);
+    sj = fmaf(__fmul_rn(fj[c], p.inv_j), e, sj);
+  }
+  const float ci = coef * p.inv_i, cj = coef * p.inv_j;
+  for (int c = 0; c < a.d; ++c) {
+    const float hi = __fmul_rn(fi[c], p.inv_i), hj = __fmul_rn(fj[c], p.inv_j);
+    const float e = fmaf(fj[c] - fi[c], inv_lo, __fmul_rn(fs[c], dinv));
+    atomicAdd(g_feats + i * a.d + c, ci * (p.clamped_i ? hj : fmaf(-si, hi, e)));
+    atomicAdd(g_feats + j * a.d + c, cj * (p.clamped_j ? hi : fmaf(sj, hj, -e)));
+  }
+}
+
+// one pair i < j of identical tuples, in both kernels: its forward statistics, or its share of the gradient
+template <bool BACKWARD>
+__device__ __forceinline__ void visit_pair(const UniqArgs& a, int64_t i, int64_t j, float coef, float* __restrict__ g_feats,
+                                           double& hinge_sum, double& pair_count, double& has_later) {
+  const PairCos p = pair_cos(a, i, j);
+  const float hinge = p.cs - a.margin;
+  if (!BACKWARD) {
+    has_later = 1.0;
+    pair_count += 1.0;
+    if (hinge > 0.f) hinge_sum += static_cast<double>(hinge);
+  } else if (hinge > 0.f && coef != 0.f) {
+    pair_grad(a, i, j, p, coef, g_feats);
+  }
 }
 
 // Keys of rows [row0, row0 + kTile) into s_keys (every thread of the CTA calls it; rows past the end get 0).  Narrow rows:
@@ -133,23 +188,7 @@ __global__ void __launch_bounds__(kTile) uniq_kernel(UniqArgs a, double* __restr
       if (s_keys[jj] != my_key) continue;
       const int64_t j = j0 + jj;
       if (j <= i || !same_tuple(a, i, j)) continue;
-      float inv_i, inv_j;
-      const float cs = pair_cos(a, i, j, &inv_i, &inv_j);
-      const float hinge = cs - a.margin;
-      if (!BACKWARD) {
-        has_later = 1.0;
-        pair_count += 1.0;
-        if (hinge > 0.f) hinge_sum += static_cast<double>(hinge);
-      } else if (hinge > 0.f && coef != 0.f) {
-        // d cos / d f_i = (fhat_j - cos * fhat_i) / |f_i|
-        const float* fi = a.feats + i * a.d;
-        const float* fj = a.feats + j * a.d;
-        for (int c = 0; c < a.d; ++c) {
-          const float hi = fi[c] * inv_i, hj = fj[c] * inv_j;
-          atomicAdd(g_feats + i * a.d + c, coef * (hj - cs * hi) * inv_i);
-          atomicAdd(g_feats + j * a.d + c, coef * (hi - cs * hj) * inv_j);
-        }
-      }
+      visit_pair<BACKWARD>(a, i, j, coef, g_feats, hinge_sum, pair_count, has_later);
     }
   }
   if (!BACKWARD) {
@@ -192,22 +231,7 @@ __global__ void __launch_bounds__(kTile) uniq_sorted_kernel(UniqArgs a, const ui
     for (int64_t q = p + 1; q < a.rows && keys[q] == my_key; ++q) {
       const int64_t j = order[q];  // (stable sort: j > i)
       if (!same_tuple(a, i, j)) continue;
-      float inv_i, inv_j;
-      const float cs = pair_cos(a, i, j, &inv_i, &inv_j);
-      const float hinge = cs - a.margin;
-      if (!BACKWARD) {
-        has_later = 1.0;
-        pair_count += 1.0;
-        if (hinge > 0.f) hinge_sum += static_cast<double>(hinge);
-      } else if (hinge > 0.f && coef != 0.f) {
-        const float* fi = a.feats + i * a.d;
-        const float* fj = a.feats + j * a.d;
-        for (int c = 0; c < a.d; ++c) {
-          const float hi = fi[c] * inv_i, hj = fj[c] * inv_j;
-          atomicAdd(g_feats + i * a.d + c, coef * (hj - cs * hi) * inv_i);
-          atomicAdd(g_feats + j * a.d + c, coef * (hi - cs * hj) * inv_j);
-        }
-      }
+      visit_pair<BACKWARD>(a, i, j, coef, g_feats, hinge_sum, pair_count, has_later);
     }
   }
   if (!BACKWARD) {
@@ -278,7 +302,7 @@ extern "C" int hv_uniq_backward(const int64_t* ids, int64_t rows, int64_t width,
                                 const float* g_out, float* g_feats, void* workspace, size_t workspace_bytes, void* stream) {
   using namespace hv;
   if (int st = check(ids, rows, width, feats, d, "hv_uniq_backward")) return st;
-  if (!stats || !g_out || (rows > 0 && !g_feats)) {
+  if (!stats || !g_out || (rows > 0 && d > 0 && !g_feats)) {
     set_error("hv_uniq_backward: null pointer");
     return HV_ERR_NULL;
   }

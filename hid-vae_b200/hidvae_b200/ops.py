@@ -391,10 +391,16 @@ def _sort_workspace(n: int, device) -> Optional[Tensor]:
 
 
 def kmeans_accumulate(x: Tensor, assign: Tensor, k: int, prev_assign: Optional[Tensor] = None):
-    """Deterministic per-cluster sums [K, D], counts [K] and the number of changed assignments (0-d int64)."""
-    _require_cuda(x, assign)
-    x = _f32c(x)
+    """Deterministic per-cluster sums [K, D], counts [K] and the number of changed assignments (0-d int64).
+    `assign` and `prev_assign` are int64 [N] with values in [0, k)."""
+    if x.dim() != 2:
+        raise ValueError("kmeans_accumulate: x must be [N, D]")
     n, d = x.shape
+    for name, a in (("assign", assign), ("prev_assign", prev_assign)):
+        if a is not None and (a.dtype != torch.int64 or tuple(a.shape) != (n,)):
+            raise ValueError(f"kmeans_accumulate: {name} must be int64 [{n}], got {a.dtype} {list(a.shape)}")
+    _require_cuda(x, assign, prev_assign)
+    x = _f32c(x)
     sums = torch.empty((k, d), dtype=torch.float32, device=x.device)
     counts = torch.empty((k,), dtype=torch.float32, device=x.device)
     changed = torch.empty((), dtype=torch.int64, device=x.device)
@@ -429,10 +435,12 @@ def kmeans_finalize(sums: Tensor, counts: Tensor, centroids: Tensor, reseed_rows
 # ------------------------------------------------------------------------------------------------------------------
 def uniq_stats(ids: Tensor, feats: Optional[Tensor], margin: float) -> Tensor:
     """stats [3] double: (sum of hinges over identical pairs i<j, number of such pairs, rows with a later twin)."""
-    _require_cuda(ids)
     if ids.dtype != torch.int64 or ids.dim() != 2:
         raise ValueError("uniq_stats: ids must be int64 [rows, width]")
     rows, width = ids.shape
+    if feats is not None and (feats.dim() != 2 or feats.shape[0] < rows):
+        raise ValueError(f"uniq_stats: feats must be [>= {rows}, D] (one row per id row), got {list(feats.shape)}")
+    _require_cuda(ids)
     d = 0
     if feats is not None:
         _require_cuda(feats)

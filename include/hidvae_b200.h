@@ -127,6 +127,9 @@ int hv_rq_backward(const float* x, int64_t n, int d, const float* codebooks, int
 /*
  * K-means codebook init (init/kmeans.py:43-61).  Assignment = hv_rq_forward with n_levels = 1 (ids only).
  * hv_kmeans_accumulate: deterministic (bit-reproducible) per-cluster sums and counts of the assigned rows
+ *   assign and prev_assign are int64 [n] and every assignment must lie in [0, K): the segmented form's search over keys
+ *   sorted on ceil(log2 K) bits assumes it, and the scan form drops other rows.  Each sum is a compensated (Kahan)
+ *   fp32 sum in a fixed order, within a few fp32 ulps of sum |x| whatever the cluster's size.
  *   sums [K, D] and counts [K] (float) are OVERWRITTEN; n_changed[0] (int64, may be NULL) receives the number
  *   of rows whose assignment differs from prev_assign (NULL = count every row).
  *   workspace: optional hv_sort_workspace_bytes(n) bytes.  With it, large K * N take the SEGMENTED form: rows are
@@ -150,7 +153,9 @@ int hv_kmeans_finalize(const float* sums, const float* counts, const float* rese
  *          stats[1] = number of such pairs, stats[2] = number of rows that have a LATER identical row.
  *          stats is OVERWRITTEN.  loss = weight * stats[0] / stats[1] (0 when stats[1] == 0) is formed by the
  *          caller on the device; p_unique = (rows - stats[2]) / rows.
- * Backward: g_feats [rows, D] (caller zeroes) += g_out[0] * weight / stats[1] * d(sum)/d feats.
+ * Backward: g_feats [rows, D] (caller zeroes) += g_out[0] * weight / stats[1] * d(sum)/d feats, in a form without
+ *          cancellation (exactly 0 for identical feature rows); a row with |f| < 1e-12 takes F.normalize's clamp
+ *          derivative.  feats has at least `rows` rows.
  * workspace: optional hv_sort_workspace_bytes(rows) bytes.  With it, batches of >= 4096 rows are key-sorted by tuple and
  *   only runs of identical tuples are walked (O(rows + pairs)); otherwise all pairs i < j are swept (O(rows^2)).
  */
