@@ -69,6 +69,12 @@ SIGNATURES = {
                                    c_void_p]),
     "hv_encoder_forward_f16": (c_int, [c_void_p, c_int64, c_int, POINTER(c_int), c_void_p, c_size_t, c_int, c_int, c_void_p,
                                        c_void_p]),
+    "hv_tag_heads_workspace_bytes": (c_size_t, [c_int, c_int, c_int, POINTER(c_int), c_int, c_int64, POINTER(c_size_t)]),
+    "hv_tag_heads_pack": (c_int, [POINTER(c_void_p), c_int, c_int, c_int, c_int, POINTER(c_int), c_int, c_void_p, c_size_t,
+                                  c_void_p]),
+    "hv_tag_heads_forward": (c_int, [c_void_p, c_int64, c_int64, c_int64, c_int, c_int, c_int, POINTER(c_int), c_int, c_void_p,
+                                     c_size_t, c_void_p, c_int64, c_int64, c_void_p, c_int64, c_int64, POINTER(c_void_p),
+                                     c_void_p, c_size_t, c_void_p]),
     "hv_peer_allreduce_chunks": (c_int, [c_int64]),
     "hv_peer_allreduce_set_timeout_ms": (None, [c_int64]),
     "hv_peer_allreduce_status": (c_int, [ctypes.c_uint32, POINTER(c_int), POINTER(c_int)]),

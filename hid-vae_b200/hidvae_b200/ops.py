@@ -6,6 +6,7 @@ a kernel in libhidvae_b200.so.  Tensors must live on a CUDA device: there is no 
 Mirrors, per function, the reference call sequence it replaces:
   rq_forward / RqFunction     modules/quantize.py:106-148 x L levels + modules/h_rqvae.py:515-523,552,572-574
   encoder_pack / encoder_forward   modules/encoder.py:23-36 (the MLP in front of the quantiser, eval passes)
+  tag_heads_pack / _forward   modules/h_rqvae.py:69-99 + :385-389 (eval TagPredictor -> argmax / confidence)
   kmeans_*                    init/kmeans.py:43-61
   uniqueness_loss / count     modules/h_rqvae.py:41-105, :645-648
   semid_dedup / merge_runs    the collision digit of HSemanticIdTokenizer(use_dedup_dim=True)
@@ -372,6 +373,78 @@ def encoder_forward(x: Tensor, image: EncoderImage, normalize: bool = False, pre
         check(fn(x.data_ptr(), n, len(dims) - 1, _dims_array(dims), image.data_ptr(), image.numel(),
                  int(bool(normalize)), int(bool(precise_silu)), z.data_ptr(), _stream(x)))
     return z
+
+
+# ------------------------------------------------------------------------------------------------------------------
+# tag heads (modules/h_rqvae.py TagPredictor, eval mode) -- inference only: training keeps the PyTorch heads
+# ------------------------------------------------------------------------------------------------------------------
+def _tag_shape_args(n_levels, d, first_hidden, class_counts, use_norm):
+    counts = (ctypes.c_int * len(class_counts))(*[int(c) for c in class_counts])
+    return int(n_levels), int(d), int(first_hidden), counts, int(bool(use_norm))
+
+
+def tag_heads_supported(n_levels: int, d: int, first_hidden: int, class_counts, use_norm: bool) -> bool:
+    """True when hv_tag_heads_forward serves this HRqVae shape (len(class_counts) must be n_levels)."""
+    if len(class_counts) != n_levels:
+        return False
+    return int(lib.hv_tag_heads_workspace_bytes(*_tag_shape_args(n_levels, d, first_hidden, class_counts, use_norm), 1,
+                                                None)) > 0
+
+
+class TagHeadsImage(NamedTuple):
+    data: Tensor          # uint8: fp16 weight blocks and fp32 biases / LayerNorm parameters of every level
+    shape: tuple          # (n_levels, d, first_hidden, class_counts, use_norm)
+
+
+def tag_heads_pack(params, d: int, first_hidden: int, class_counts, use_norm: bool) -> TagHeadsImage:
+    """Image of the tag heads (hv_tag_heads_pack).  `params`: every level's TagPredictor.parameters(), level by level."""
+    params = [_f32c(p.detach()) for p in params]
+    _require_cuda(*params)
+    n_levels = len(class_counts)
+    shape = _tag_shape_args(n_levels, d, first_hidden, class_counts, use_norm)
+    nbytes = ctypes.c_size_t(0)
+    if not int(lib.hv_tag_heads_workspace_bytes(*shape, 1, ctypes.byref(nbytes))):
+        raise _lib.HidvaeError(_lib.HV_ERR_UNSUPPORTED, f"no tag-head instantiation for L={n_levels}, D={d}, "
+                               f"hidden={first_hidden}, classes={list(class_counts)}")
+    image = torch.empty(nbytes.value, dtype=torch.uint8, device=params[0].device)
+    ptrs = (ctypes.c_void_p * len(params))(*[p.data_ptr() for p in params])
+    with torch.cuda.device(image.device):
+        check(lib.hv_tag_heads_pack(ptrs, len(params), *shape, image.data_ptr(), nbytes.value, _stream(image)))
+    return TagHeadsImage(image, (n_levels, int(d), int(first_hidden), tuple(int(c) for c in class_counts), bool(use_norm)))
+
+
+def tag_heads_forward(emb: Tensor, image: TagHeadsImage, pred_out: Optional[Tensor] = None,
+                      conf_out: Optional[Tensor] = None, logits_out=None):
+    """(pred [N, L] int64, conf [N, L] fp32 or None) of the tag heads on level embeddings emb [L, N, D] fp32 (any strides
+    with a contiguous last dimension).  `pred_out` / `conf_out` may be strided [N, L] views -- e.g. the tag columns of an
+    id table -- and are written in place; `logits_out` is an optional list of L fp32 [N, C_i] tensors."""
+    n_levels, d, first_hidden, counts, use_norm = image.shape
+    _require_cuda(emb, image.data)
+    if emb.dtype != torch.float32 or emb.dim() != 3 or emb.shape[0] < n_levels or emb.shape[2] != d or emb.stride(2) != 1:
+        raise ValueError(f"tag_heads_forward: emb must be fp32 [>= {n_levels}, N, {d}] with a contiguous last dimension, "
+                         f"got {emb.dtype} {tuple(emb.shape)}")
+    n = emb.shape[1]
+    if pred_out is None:
+        pred_out = torch.empty((n, n_levels), dtype=torch.int64, device=emb.device)
+    for name, t, dt in (("pred_out", pred_out, torch.int64), ("conf_out", conf_out, torch.float32)):
+        if t is not None and (t.dtype != dt or t.shape != (n, n_levels) or t.device != emb.device):
+            raise ValueError(f"tag_heads_forward: {name} must be {dt} [{n}, {n_levels}] on {emb.device}")
+    logit_ptrs = None
+    if logits_out is not None:
+        for t, c in zip(logits_out, counts):
+            if t.dtype != torch.float32 or t.shape != (n, c) or not t.is_contiguous():
+                raise ValueError(f"tag_heads_forward: logits_out entries must be contiguous fp32 [{n}, C_i]")
+        logit_ptrs = (ctypes.c_void_p * n_levels)(*[t.data_ptr() for t in logits_out])
+    shape = _tag_shape_args(n_levels, d, first_hidden, counts, use_norm)
+    ws_bytes = int(lib.hv_tag_heads_workspace_bytes(*shape, n, None))
+    workspace = torch.empty(ws_bytes, dtype=torch.uint8, device=emb.device)
+    with torch.cuda.device(emb.device):
+        check(lib.hv_tag_heads_forward(
+            emb.data_ptr(), emb.stride(0), emb.stride(1), n, *shape, image.data.data_ptr(), image.data.numel(),
+            pred_out.data_ptr(), pred_out.stride(0), pred_out.stride(1),
+            _ptr(conf_out), conf_out.stride(0) if conf_out is not None else 0, conf_out.stride(1) if conf_out is not None else 0,
+            logit_ptrs, workspace.data_ptr(), ws_bytes, _stream(emb)))
+    return pred_out, conf_out
 
 
 # ------------------------------------------------------------------------------------------------------------------

@@ -146,6 +146,10 @@ class HRqVae(nn.Module, _HubMixin):
         self.sem_id_uniqueness_weight = sem_id_uniqueness_weight
         self.uniqueness_as_reference = True   # transposed-ids call of h_rqvae.py:630-631 (see module docstring)
         self.fuse_levels = True               # False forces the reference's level-by-level loop
+        # "torch": predict_tags runs the PyTorch heads; "fused": eval-mode, no-grad CUDA calls of a served shape run the
+        # tcgen05 tag-head kernels (csrc/tag_heads.cu: fp16 operands, fp32 accumulation); training always uses PyTorch
+        self.tag_inference_precision = "torch"
+        self._tag_image, self._tag_image_key = None, None
 
         self.tag_class_counts = ([10, 100, 1000] if tag_class_counts is None else list(tag_class_counts))[:n_layers]
         assert len(self.tag_class_counts) == n_layers, (
@@ -370,6 +374,52 @@ class HRqVae(nn.Module, _HubMixin):
             tag_align_loss_by_layer=q.tag_align_loss_by_layer, tag_pred_loss_by_layer=q.tag_pred_loss_by_layer,
             tag_pred_accuracy_by_layer=q.tag_pred_accuracy_by_layer, sem_id_uniqueness_loss=uniqueness)
 
+    def _tag_heads_shape(self):
+        """(d, first_hidden, class_counts, use_norm) when the heads have the architecture the fused kernels compute."""
+        first_hidden, counts, norms = self.hidden_dims[0], [], []
+        for i, tp in enumerate(self.tag_predictors):
+            fe, cl = tp.feature_extractor, tp.classifier
+            lns = [m for m in tp.modules() if isinstance(m, nn.LayerNorm)]
+            if (tp.attention[0].in_features != self.embed_dim * (i + 1) or fe[0].out_features != first_hidden // 2 * (i + 1)
+                    or tp.apply_norm != (i > 0) or any(m.eps != 1e-5 or not m.elementwise_affine for m in lns)):
+                return None
+            norms.append(isinstance(fe[1], nn.LayerNorm))
+            counts.append(cl[-1].out_features)
+        if len(set(norms)) != 1 or not ops.tag_heads_supported(self.n_layers, self.embed_dim, first_hidden, counts, norms[0]):
+            return None
+        return self.embed_dim, first_hidden, counts, norms[0]
+
+    def _fused_tag_image(self, level_embeddings: Tensor):
+        """The packed tag-head image when this call takes the fused path, else None.  Re-packed whenever a weight
+        changed (version counters), like MLP._weight_image."""
+        if self.tag_inference_precision not in ("torch", "fused"):
+            raise ValueError(f"tag_inference_precision must be 'torch' or 'fused', got {self.tag_inference_precision!r}")
+        if (self.tag_inference_precision != "fused" or not level_embeddings.is_cuda or torch.is_grad_enabled()
+                or any(m.training for m in self.tag_predictors.modules())):
+            return None
+        shape = self._tag_heads_shape()
+        if shape is None:
+            return None
+        params = [p for tp in self.tag_predictors for p in tp.parameters()]
+        key = (tuple(shape[2]), shape[3], tuple((p.data_ptr(), p._version) for p in params))
+        if self._tag_image is None or key != self._tag_image_key:
+            self._tag_image, self._tag_image_key = ops.tag_heads_pack(params, *shape), key
+        return self._tag_image
+
+    def predict_tags_into(self, level_embeddings: Tensor, pred_out: Optional[Tensor],
+                          conf_out: Optional[Tensor] = None) -> bool:
+        """Fused path only: write the predicted tags of level_embeddings [L, N, D] into pred_out [N, L] int64 (any
+        strides, e.g. the tag columns of an id table) and return True; False (nothing written) when the call does not
+        take the fused path."""
+        if pred_out is None:
+            return False
+        image = self._fused_tag_image(level_embeddings)
+        if image is None:
+            return False
+        emb = level_embeddings.float()
+        ops.tag_heads_forward(emb if emb.stride(-1) == 1 else emb.contiguous(), image, pred_out, conf_out)
+        return True
+
     def predict_tags(self, x: Tensor, gumbel_t: float = 0.001, encoded: Optional[Tensor] = None,
                      level_embeddings: Optional[Tensor] = None) -> Dict[str, Tensor]:
         """Tag ids + confidences per level for x [B, F] or [B, S, F] (reference h_rqvae.py:674-738).  Passing
@@ -382,6 +432,14 @@ class HRqVae(nn.Module, _HubMixin):
         if level_embeddings is None:
             enc = self.encode(x) if encoded is None else encoded
             level_embeddings, _res, _ids, _loss = self.quantize_all_levels(enc, gumbel_t)
+        if self._fused_tag_image(level_embeddings) is not None:
+            n = level_embeddings.shape[1]
+            pred = torch.empty((n, self.n_layers), dtype=torch.int64, device=level_embeddings.device)
+            conf = torch.empty((n, self.n_layers), dtype=torch.float32, device=level_embeddings.device)
+            self.predict_tags_into(level_embeddings, pred, conf)
+            if seq:
+                pred, conf = pred.reshape(shape[0], shape[1], -1), conf.reshape(shape[0], shape[1], -1)
+            return {"predictions": pred, "confidences": conf}
         preds, confs = [], []
         for i in range(self.n_layers):
             concat = torch.cat(list(level_embeddings[: i + 1]), dim=-1)

@@ -36,6 +36,14 @@ def _features_of(dataset, lo: int, hi: int) -> Tensor:
     return torch.stack([r if isinstance(r, Tensor) else torch.as_tensor(r) for r in rows])
 
 
+def _column_view(rows: Tensor, cols: List[int]) -> Optional[Tensor]:
+    """rows[:, cols] as a strided view when the columns are evenly spaced (the concatenated and interleaved layouts)."""
+    step = cols[1] - cols[0] if len(cols) > 1 else 1
+    if step < 1 or cols != list(range(cols[0], cols[0] + step * len(cols), step)):
+        return None
+    return rows[:, cols[0]: cols[-1] + 1: step]
+
+
 class HSemanticIdTokenizer(nn.Module):
     def __init__(
         self,
@@ -58,6 +66,7 @@ class HSemanticIdTokenizer(nn.Module):
         use_interleaved_ids: bool = False,
         chunk_items: int = 1 << 18,
         encoder_precision: str = "fused",
+        tag_precision: str = "torch",
     ) -> None:
         super().__init__()
         if sum(map(bool, (use_dedup_dim, use_concatenated_ids, use_interleaved_ids))) > 1:
@@ -79,6 +88,9 @@ class HSemanticIdTokenizer(nn.Module):
             self.hrq_vae.load_pretrained(hrqvae_weights_path)
         self.hrq_vae.eval()
         self.hrq_vae.encoder.inference_precision = encoder_precision
+        # tag_precision (HRqVae.tag_inference_precision): "torch" = the PyTorch tag heads; "fused" = the tcgen05 tag-head
+        # kernels (fp16 operands, fp32 accumulation), which write the predicted tags straight into their id-table columns
+        self.hrq_vae.tag_inference_precision = tag_precision
         self.codebook_size = codebook_size
         self.n_layers = n_layers
         self.use_dedup_dim = use_dedup_dim
@@ -162,7 +174,9 @@ class HSemanticIdTokenizer(nn.Module):
                 level_emb, _res, ids, _loss = model.quantize_all_levels(enc)
             if not (fused and contiguous_sem):
                 rows[:, sem_cols] = ids
-            if tag_cols:
+            if tag_cols and model.predict_tags_into(level_emb, _column_view(rows, tag_cols)):
+                pass  # the fused heads wrote the tag columns in place
+            elif tag_cols:
                 tags = model.predict_tags(x, level_embeddings=level_emb)["predictions"]
                 if tags.shape[0] != ids.shape[0]:
                     raise ValueError(f"Semantic ID batch size ({ids.shape[0]}) does not match predicted tag batch size ({tags.shape[0]})")
@@ -255,7 +269,7 @@ class HSemanticIdTokenizer(nn.Module):
         level_emb, _res, ids, _loss = model.quantize_all_levels(enc)
         rows = torch.empty((x.shape[0], len(sem_cols) + len(tag_cols)), dtype=torch.int64, device=ids.device)
         rows[:, sem_cols] = ids
-        if tag_cols:
+        if tag_cols and not model.predict_tags_into(level_emb, _column_view(rows, tag_cols)):
             rows[:, tag_cols] = model.predict_tags(x, level_embeddings=level_emb)["predictions"]
         return rows
 

@@ -145,6 +145,8 @@ def train(
     uniqueness_as_reference=True,
     use_cuda_graph=False,      # replay the micro-step (gather + forward + backward) and the AdamW step as CUDA graphs
                                # (hidvae_b200/graph_step.py); not with fp16 loss scaling
+    tag_precision="torch",     # tag heads of the eval catalogue pass: "torch" (the PyTorch heads) or "fused"
+                               # (the tcgen05 kernels of csrc/tag_heads.cu, HRqVae.tag_inference_precision)
 ):
     rank, world, local = hv_dist.init_from_env()
     is_main = rank == 0
@@ -271,8 +273,9 @@ def train(
             tag_alignment_weight=tag_alignment_weight, tag_prediction_weight=tag_prediction_weight,
             tag_class_counts=model.tag_class_counts, tag_embed_dim=tag_embed_dim,
             use_concatenated_ids=use_concatenated_ids, use_interleaved_ids=use_interleaved_ids,
-            commitment_weight=commitment_weight)
+            commitment_weight=commitment_weight, tag_precision=tag_precision)
         tokenizer.hrq_vae = model
+        model.tag_inference_precision = tag_precision
 
         # running sums of the logged quantities live on the device; .tolist() happens only when a line is printed
         names = ["loss", "reconstruction", "rqvae", "tag_align", "tag_pred", "tag_acc", "p_unique"]

@@ -263,6 +263,37 @@ int hv_encoder_forward_f16(const void* x_f16, int64_t n, int n_layers, const int
                            int normalize, int precise_silu, float* z, void* stream);
 
 /*
+ * Eval-mode tag heads: per level i the TagPredictor of modules/h_rqvae.py:69-99 (reference h_rqvae.py:108-227) on
+ * concat(emb_0 .. emb_i), reduced to argmax and softmax confidence as predict_tags does (reference h_rqvae.py:674-738).
+ * The attention gate runs in fp32 on CUDA cores; every Linear after it is a tcgen05 GEMM with fp16 operands (the
+ * encoder's numerics), fp32 accumulation, fp32 LayerNorm statistics / softmax / argmax (first index on ties).  Inference
+ * only: dropout is the identity and LayerNorm uses its affine parameters.
+ *   n_levels, d, first_hidden, class_counts, use_norm   the HRqVae shape: level i has E = d (i+1) inputs, hidden width
+ *               H = first_hidden / 2 (i+1), inner width int(0.9 H), class_counts[i] (HOST array) classes; use_norm = 1 when
+ *               the heads were built with use_batch_norm=True (nn.LayerNorm), 0 for nn.Identity.  Served: n_levels <= 8,
+ *               E <= 128, padded widths <= 4096; otherwise HV_ERR_UNSUPPORTED / a zero size (the caller keeps PyTorch).
+ * hv_tag_heads_workspace_bytes  scratch bytes hv_tag_heads_forward needs for `rows` rows (it works on sub-chunks of at
+ *               most 18,944 rows, so the size stops growing there); *image_bytes (nullable) receives the image size.
+ * hv_tag_heads_pack  params = HOST array of DEVICE fp32 pointers, level by level in TagPredictor.parameters() order
+ *               (34 per level with LayerNorm, 22 without); writes the image once per set of weights.
+ * hv_tag_heads_forward
+ *   emb         level embeddings, element (l, r, c) at emb[l * emb_level_stride + r * emb_row_stride + c] (fp32)
+ *   pred_out    int64, level i of row r at pred_out[r * pred_row_stride + i * pred_level_stride] (e.g. the tag columns of
+ *               an id table); conf_out (nullable) fp32 the same way
+ *   logits_out  nullable HOST array of n_levels nullable DEVICE pointers: fp32 [n, class_counts[i]] logits of level i
+ * Nothing else of pred_out / conf_out is written.
+ */
+size_t hv_tag_heads_workspace_bytes(int n_levels, int d, int first_hidden, const int* class_counts, int use_norm, int64_t rows,
+                                    size_t* image_bytes);
+int hv_tag_heads_pack(const float* const* params, int n_params, int n_levels, int d, int first_hidden, const int* class_counts,
+                      int use_norm, void* image, size_t image_bytes, void* stream);
+int hv_tag_heads_forward(const float* emb, int64_t emb_level_stride, int64_t emb_row_stride, int64_t n, int n_levels, int d,
+                         int first_hidden, const int* class_counts, int use_norm, const void* image, size_t image_bytes,
+                         int64_t* pred_out, int64_t pred_row_stride, int64_t pred_level_stride, float* conf_out,
+                         int64_t conf_row_stride, int64_t conf_level_stride, float* const* logits_out, void* workspace,
+                         size_t workspace_bytes, void* stream);
+
+/*
  * Data-parallel exchange of a small fp32 buffer (the codebook gradient, train_hidvae.py's DDP all-reduce) as ONE kernel
  * over NVLink / NVSwitch peer memory: every rank pushes its contribution into an inbox slot on every peer, flags it,
  * waits for its peers' flags and sums the slots in rank order (bit-identical results on every rank).
