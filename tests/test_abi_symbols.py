@@ -6,17 +6,9 @@ import re
 
 import pytest
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+from helpers import ROOT, lib_mod
+
 HEADER = os.path.join(ROOT, "include", "hidvae_b200.h")
-
-
-@pytest.fixture(scope="module")
-def lib_mod():
-    import __graft_entry__ as g
-    if not os.path.isfile(os.path.join(ROOT, "hid-vae_b200", "libhidvae_b200.so")):
-        g.build()
-    from hidvae_b200 import _lib
-    return _lib
 
 
 def _declared_symbols():

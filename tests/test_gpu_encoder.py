@@ -10,19 +10,13 @@ import pytest
 import torch
 import torch.nn.functional as F
 
-from helpers import make_codebooks, npz, t
+from helpers import make_codebooks, npz, ops, t
 from oracle import encoder as OE
 from oracle import rq as O
 
 pytestmark = pytest.mark.gpu
 DIMS = [768, 512, 256, 128, 32]
 TOL = 2e-3
-
-
-@pytest.fixture(scope="module")
-def ops():
-    from hidvae_b200 import ops as _ops
-    return _ops
 
 
 @pytest.fixture(scope="module")

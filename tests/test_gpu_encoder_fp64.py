@@ -36,23 +36,19 @@ Each cell asserts under torch.profiler which instantiation ran; test_every_shipp
 library with cuobjdump and fails when an instantiation has no cell.
 """
 import functools
-import os
-import re
-import shutil
-import subprocess
 
 import numpy as np
 import pytest
 import torch
 import torch.nn.functional as F
 
+from helpers import assert_launched, family, ops, profiled, shipped_kernels
 from oracle import encoder as OE
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-LIB = os.path.join(ROOT, "hid-vae_b200", "libhidvae_b200.so")
 DIMS = [768, 512, 256, 128, 32]
 F16_MAX = 65504.0
 SUBNORMALS_KEPT = True
+FAMILIES = ("enc_mlp_kernel",)
 KERNELS = {(p, h): f"enc_mlp_kernel<{'true' if p else 'false'},{'true' if h else 'false'}>" for p in (0, 1) for h in (0, 1)}
 N_STAT = 148 * 128 + 77                       # every CTA busy, a ragged last tile
 WITHIN = 1e-5
@@ -75,12 +71,6 @@ BARS = {
     ("subnormal", 0, 0): (1.4e-3, 1.2e-4, 0.38),   # 6.89e-4, 5.86e-5, 0.768
     ("subnormal", 0, 1): (1.5e-3, 1.2e-4, 0.38),   # 7.66e-4, 6.00e-5, 0.768
 }
-
-
-@pytest.fixture(scope="module")
-def ops():
-    from hidvae_b200 import ops as _ops
-    return _ops
 
 
 # ---------------------------------------------------------------------------------------------------------------------
@@ -202,49 +192,13 @@ def exact_z(x, weights, normalize):
     return exact_tail(z64) if normalize else z64.float()
 
 
-# ---------------------------------------------------------------------------------------------------------------------
-# kernel names: torch.profiler (demangled) and cuobjdump (mangled)
-# ---------------------------------------------------------------------------------------------------------------------
-_DEMANGLED = re.compile(r"\benc_mlp_kernel<([^<>]*)>")
-_MANGLED = re.compile(r"\denc_mlp_kernelI((?:Lb\dE)+)E")
-
-
-def normalise(name):
-    m = _DEMANGLED.search(name)
-    if m is None:
-        return None
-    args = [a.strip().replace("(bool)1", "true").replace("(bool)0", "false") for a in m.group(1).split(",")]
-    return f"enc_mlp_kernel<{','.join(args)}>"
-
-
-def shipped_instantiations(symbols_text):
-    return {"enc_mlp_kernel<" + ",".join("true" if v == "1" else "false" for v in re.findall(r"Lb(\d)E", args)) + ">"
-            for args in _MANGLED.findall(symbols_text)}
-
-
-def profiled(fn):
-    """fn() once under torch.profiler; returns (result, set of enc_mlp_kernel instantiations launched, any CUDA kernel seen)."""
-    from torch.profiler import ProfilerActivity, profile
-    torch.cuda.synchronize()
-    with profile(activities=[ProfilerActivity.CPU, ProfilerActivity.CUDA]) as prof:
-        result = fn()
-        torch.cuda.synchronize()
-    names, recorded = set(), False
-    for ev in prof.events():
-        recorded |= ev.device_type == torch.autograd.DeviceType.CUDA
-        n = normalise(ev.name)
-        if n is not None:
-            names.add(n)
-    return result, names, recorded
-
-
 def run_cell(ops, x, image, precise, half_in, normalize, **kw):
     """encoder_forward under the profiler; asserts that exactly the expected instantiation ran."""
     xin = x.half() if half_in else x
-    z, names, recorded = profiled(lambda: ops.encoder_forward(xin, image, normalize=bool(normalize),
-                                                              precise_silu=bool(precise), **kw))
-    assert recorded, "torch.profiler recorded no CUDA kernel"
-    assert names == {KERNELS[(precise, half_in)]}, f"expected {KERNELS[(precise, half_in)]}, launched {sorted(names)}"
+    z, launches = profiled(lambda: ops.encoder_forward(xin, image, normalize=bool(normalize), precise_silu=bool(precise),
+                                                       **kw))
+    assert launches.recorded, "torch.profiler recorded no CUDA kernel"
+    assert_launched(launches, {KERNELS[(precise, half_in)]}, FAMILIES)
     return z
 
 
@@ -338,24 +292,9 @@ def test_integer_network_is_exact_and_the_tail_is_fp32_normalize():
         torch.testing.assert_close(tail.double(), F.normalize(zz, dim=-1, eps=1e-12), rtol=0, atol=4e-7)
 
 
-def test_kernel_name_normalisation():
-    assert normalise("void hv::(anonymous namespace)::enc_mlp_kernel<(bool)1, (bool)0>(hv::(anonymous namespace)::EncArgs)") \
-        == "enc_mlp_kernel<true,false>"
-    assert normalise("void hv::(anonymous namespace)::enc_mlp_kernel<true, true>(hv::(anonymous namespace)::EncArgs)") \
-        == "enc_mlp_kernel<true,true>"
-    assert shipped_instantiations("_ZN2hv43_GLOBAL__N__053ced98_10_enc_mlp_cu_09e2636814enc_mlp_kernelILb0ELb1EEEvNS0_7EncArgsE") \
-        == {"enc_mlp_kernel<false,true>"}
-
-
 def test_every_shipped_instantiation_has_a_cell():
     """Every enc_mlp_kernel instantiation in the built library is the expected kernel of some cell (cuobjdump, CPU only)."""
-    tool = shutil.which("cuobjdump") or os.path.join(os.environ.get("CUDA_HOME", "/usr/local/cuda"), "bin", "cuobjdump")
-    if not os.path.isfile(LIB):
-        pytest.skip(f"{os.path.relpath(LIB, ROOT)} is not built")
-    if not os.path.isfile(tool):
-        pytest.skip("cuobjdump not found")
-    text = subprocess.run([tool, "-symbols", LIB], check=True, capture_output=True, text=True).stdout
-    shipped = shipped_instantiations(text)
+    shipped = {k for k in shipped_kernels() if family(k) in FAMILIES}
     covered = {KERNELS[(p, h)] for p, h, _ in instantiation_cells()}
     assert shipped, "no enc_mlp_kernel in the library"
     assert not sorted(shipped - covered), f"shipped instantiations without a cell: {sorted(shipped - covered)}"

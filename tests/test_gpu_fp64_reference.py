@@ -22,21 +22,14 @@ Bars (those of tests/test_gpu_rq.py and tests/test_gpu_gumbel.py; the measured w
   * codebook gradient: rtol 1e-4, atol 1e-5 x max(1, |g_cb|max)   (fp32 sums of ~N / K terms in atomic order)
 """
 import math
-import os
-import re
-import shutil
-import subprocess
 from typing import NamedTuple, Optional
 
 import pytest
 import torch
 import torch.nn.functional as F
 
-from helpers import NEAR_TIE_REL, make_codebooks, unit_rows
+from helpers import NEAR_TIE_REL, assert_launched, family, make_codebooks, ops, profiled, shipped_kernels, unit_rows
 from oracle import rq as O
-
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-LIB = os.path.join(ROOT, "hid-vae_b200", "libhidvae_b200.so")
 
 STE, ROT = O.MODE_STE, O.MODE_ROTATION_TRICK
 MODES = {"ste": (STE, True), "rot": (ROT, True), "eval": (STE, False)}   # name -> (mode, training)
@@ -52,12 +45,6 @@ FAMILIES = ("rq_bwd_kernel", "rq_bwd_smem_kernel", "rq_fwd_simt_kernel", "rq_fwd
 BWD_FAMILY = ("rq_bwd_kernel", "rq_bwd_smem_kernel")
 FWD_FAMILY = ("rq_fwd_simt_kernel", "rq_fwd_tc_kernel", "rq_fwd_tc_v11_kernel")
 GUMBEL_FAMILY = ("gumbel_fwd_kernel", "gumbel_bwd_kernel")
-
-
-@pytest.fixture(scope="module")
-def ops():
-    from hidvae_b200 import ops as _ops
-    return _ops
 
 
 # ---------------------------------------------------------------------------------------------------------------------
@@ -189,66 +176,6 @@ def grad_ratios(g_x, g_cb, ref, rows=None):
     gx = g_x if rows is None else g_x[rows]
     return {"g_x": ratio(gx, rx, GX[0], GX[1] * max(1.0, float(rx.abs().max()))),
             "g_codebooks": ratio(g_cb, ref.g_cb, GCB[0], GCB[1] * max(1.0, float(ref.g_cb.abs().max())))}
-
-
-# ---------------------------------------------------------------------------------------------------------------------
-# kernel names: torch.profiler (demangled) and cuobjdump (mangled), normalised to family<arg,arg,...>
-# ---------------------------------------------------------------------------------------------------------------------
-_DEMANGLED = re.compile(r"\b(" + "|".join(FAMILIES) + r")<([^<>]*)>")
-_MANGLED = re.compile(r"\d(" + "|".join(FAMILIES) + r")I((?:L[ib]-?\d+E)+)E")
-
-
-def _norm_arg(a):
-    a = a.strip().replace(" ", "")
-    m = re.fullmatch(r"\((bool|int)\)(-?\d+)", a)
-    if m:
-        return ("true" if m.group(2) != "0" else "false") if m.group(1) == "bool" else m.group(2)
-    return a
-
-
-def normalise(name):
-    m = _DEMANGLED.search(name)
-    return None if m is None else f"{m.group(1)}<{','.join(_norm_arg(a) for a in m.group(2).split(','))}>"
-
-
-def shipped_instantiations(symbols_text):
-    out = set()
-    for fam, args in _MANGLED.findall(symbols_text):
-        vals = [("true" if v != "0" else "false") if t == "b" else v for t, v in re.findall(r"L([ib])(-?\d+)E", args)]
-        out.add(f"{fam}<{','.join(vals)}>")
-    return out
-
-
-class Launches(NamedTuple):
-    names: set        # normalised instantiations of FAMILIES that were launched
-    recorded: bool    # the profiler recorded at least one CUDA kernel
-
-
-def profiled(fn):
-    """Run fn() once under torch.profiler (CPU + CUDA activity); returns (fn's result, Launches)."""
-    from torch.profiler import ProfilerActivity, profile
-    torch.cuda.synchronize()
-    with profile(activities=[ProfilerActivity.CPU, ProfilerActivity.CUDA]) as prof:
-        result = fn()
-        torch.cuda.synchronize()
-    names, recorded = set(), False
-    for ev in prof.events():
-        if ev.device_type == torch.autograd.DeviceType.CUDA:
-            recorded = True
-        n = normalise(ev.name)
-        if n is not None:
-            names.add(n)
-    return result, Launches(names, recorded)
-
-
-def assert_launched(launches, expected, family):
-    """`expected` (a set of instantiations) ran, and no other kernel of `family`.  Returns the skip reason when the
-    profiler saw no CUDA kernel at all (the caller skips after its numeric checks)."""
-    if not launches.recorded:
-        return "torch.profiler recorded no CUDA kernel on this machine: kernel-name assertion not possible (numbers checked)"
-    seen = {n for n in launches.names if n.split("<")[0] in family}
-    assert seen == set(expected), f"expected exactly {sorted(expected)} of {family}, launched {sorted(seen)}"
-    return None
 
 
 # ---------------------------------------------------------------------------------------------------------------------
@@ -431,38 +358,19 @@ def test_backward_nine_levels_is_unsupported_without_a_launch(ops):
             ops.rq_backward(x, cbs, ids, STE, True, BETA, None, torch.ones(100, device="cuda"), None)
 
     _, launches = profiled(call)
-    assert not {n for n in launches.names if n.split("<")[0] in BWD_FAMILY}
+    assert not {n for n in launches.names if family(n) in BWD_FAMILY}
 
 
 def test_every_shipped_instantiation_has_a_cell():
     """Every instantiation of the quantiser and Gumbel kernels in the built library is the expected kernel of some cell of
     this file (CPU only: reads the library with cuobjdump)."""
-    tool = shutil.which("cuobjdump") or os.path.join(os.environ.get("CUDA_HOME", "/usr/local/cuda"), "bin", "cuobjdump")
-    if not os.path.isfile(LIB):
-        pytest.skip(f"{os.path.relpath(LIB, ROOT)} is not built")
-    if not os.path.isfile(tool):
-        pytest.skip("cuobjdump not found")
-    text = subprocess.run([tool, "-symbols", LIB], check=True, capture_output=True, text=True).stdout
-    shipped = shipped_instantiations(text)
-    assert {s.split("<")[0] for s in shipped} == set(FAMILIES), sorted(shipped)
+    shipped = {k for k in shipped_kernels() if family(k) in FAMILIES}
+    assert {family(s) for s in shipped} == set(FAMILIES), sorted(shipped)
     covered = {c.kernel for c in BWD_CELLS + FWD_CELLS}
     covered |= {f"{fam}<{d}>" for fam in GUMBEL_FAMILY for d, _ in GUMBEL_SHAPES}
     unreached = sorted(shipped - covered)
     assert not unreached, f"{len(unreached)} of {len(shipped)} shipped instantiations have no test cell: {unreached}"
     assert not sorted(covered - shipped), f"cells expect kernels the library does not ship: {sorted(covered - shipped)}"
-
-
-def test_kernel_name_normalisation():
-    assert normalise("void hv::(anonymous namespace)::rq_bwd_smem_kernel<(int)32, (int)8, (bool)1, (bool)1, (int)3>"
-                     "(hv::(anonymous namespace)::RqBwdArgs)") == "rq_bwd_smem_kernel<32,8,true,true,3>"
-    assert normalise("void hv::(anonymous namespace)::rq_bwd_kernel<32, false, true, 0>(hv::RqBwdArgs)") == \
-        "rq_bwd_kernel<32,false,true,0>"
-    assert normalise("void hv::rq_fwd_tc_v11_kernel<false, true>(hv::RqFwdArgs, hv::V11Params)") == \
-        "rq_fwd_tc_v11_kernel<false,true>"
-    assert normalise("void at::native::vectorized_elementwise_kernel<4, float>(int)") is None
-    assert shipped_instantiations("_ZN2hv12_GLOBAL__N_118rq_bwd_smem_kernelILi32ELi8ELb1ELb1ELi3EEEvNS0_9RqBwdArgsE "
-                                  "_ZN2hv12_GLOBAL__N_113rq_bwd_kernelILi4ELb0ELb0ELi0EEEvNS0_9RqBwdArgsE") == \
-        {"rq_bwd_smem_kernel<32,8,true,true,3>", "rq_bwd_kernel<4,false,false,0>"}
 
 
 @pytest.mark.parametrize("mname", ["ste", "rot", "eval"])

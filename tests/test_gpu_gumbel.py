@@ -8,16 +8,10 @@ import numpy as np
 import pytest
 import torch
 
-from helpers import npz, t, unit_rows
+from helpers import npz, ops, t, unit_rows
 from oracle import rq as O
 
 pytestmark = pytest.mark.gpu
-
-
-@pytest.fixture(scope="module")
-def ops():
-    from hidvae_b200 import ops as _ops
-    return _ops
 
 
 def test_gumbel_golden_recorded_noise(ops, golden_dir):

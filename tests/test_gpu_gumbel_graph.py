@@ -10,37 +10,20 @@ csrc/gumbel.cu) and the seed that `ops.gumbel_apply` draws on the device while a
   trainer with use_cuda_graph = True."""
 import os
 import re
-import shutil
 import subprocess
 
 import numpy as np
 import pytest
 import torch
 
-from helpers import unit_rows
+from helpers import ROOT, family, lib_mod, ops, shipped_kernels, unit_rows
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 PKG = os.path.join(ROOT, "hid-vae_b200")
-LIB = os.path.join(PKG, "libhidvae_b200.so")
 NEW_ENTRIES = ("hv_gumbel_uniforms_devrng", "hv_gumbel_forward_devrng", "hv_gumbel_backward_devrng")
 SEED, OFFSET = 0x2F3A5B7C9D1E4F60, (1 << 33) + 12345      # the offset carries into the counter's high word
 CB_BAR = dict(rtol=1e-4)                                  # g_codebook: + atol 1e-5 x its scale (tests/test_gpu_gumbel.py)
-KERNEL = r"(gumbel_(?:fwd|bwd|uniforms)_kernel(?:ILi\d+EE)?)"
-
-
-@pytest.fixture(scope="module")
-def lib_mod():
-    import __graft_entry__ as g
-    if not os.path.isfile(LIB):
-        g.build()
-    from hidvae_b200 import _lib
-    return _lib
-
-
-@pytest.fixture(scope="module")
-def ops(lib_mod):
-    from hidvae_b200 import ops as _ops
-    return _ops
+FAMILIES = ("gumbel_fwd_kernel", "gumbel_bwd_kernel", "gumbel_uniforms_kernel")
+KERNEL = r"(gumbel_(?:fwd|bwd|uniforms)_kernel(?:ILi\d+EE)?)"                # mangled, as -Xptxas -v prints it
 
 
 def _cb_close(a, b):
@@ -89,18 +72,10 @@ def test_ops_reject_a_malformed_tensor_seed(ops, seed):
         ops.gumbel_uniforms(4, 64, seed)
 
 
-def _gumbel_symbols():
-    tool = shutil.which("cuobjdump") or os.path.join(os.environ.get("CUDA_HOME", "/usr/local/cuda"), "bin", "cuobjdump")
-    if not os.path.isfile(tool):
-        pytest.skip("cuobjdump not found")
-    text = subprocess.run([tool, "-symbols", LIB], check=True, capture_output=True, text=True).stdout
-    return set(re.findall(KERNEL, text))
-
-
 def test_same_gumbel_kernel_instantiations(lib_mod):
     """The device pair is a runtime pointer: the library ships the Gumbel instantiations it shipped before."""
-    assert _gumbel_symbols() == {f"gumbel_{f}_kernelILi{d}EE" for f in ("fwd", "bwd") for d in (16, 32, 64)} | \
-        {"gumbel_uniforms_kernel"}
+    assert {k for k in shipped_kernels() if family(k) in FAMILIES} == \
+        {f"gumbel_{f}_kernel<{d}>" for f in ("fwd", "bwd") for d in (16, 32, 64)} | {"gumbel_uniforms_kernel"}
 
 
 def test_gumbel_kernels_spill_no_more_than_before(tmp_path):

@@ -7,17 +7,11 @@ import numpy as np
 import pytest
 import torch
 
-from helpers import npz, t, unit_rows
+from helpers import npz, ops, t, unit_rows
 from oracle import kmeans as OK
 from oracle import rq as O
 
 pytestmark = pytest.mark.gpu
-
-
-@pytest.fixture(scope="module")
-def ops():
-    from hidvae_b200 import ops as _ops
-    return _ops
 
 
 def _lloyd_gpu(ops, x, init_idx, max_iters=500):

@@ -41,10 +41,6 @@ lists the shipped kernels with cuobjdump (CPU) and fails when one has no cell.
 """
 import ctypes
 import math
-import os
-import re
-import shutil
-import subprocess
 from typing import NamedTuple
 
 import numpy as np
@@ -52,12 +48,10 @@ import pytest
 import torch
 import torch.nn.functional as F
 
-from helpers import NEAR_TIE_REL, unit_rows
+from helpers import NEAR_TIE_REL, assert_launched, family, lib_mod, ops, profiled, shipped_kernels, unit_rows
 from oracle import kmeans as OK
 from oracle import rq as O
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-LIB = os.path.join(ROOT, "hid-vae_b200", "libhidvae_b200.so")
 gpu = pytest.mark.gpu
 
 U = 2.0 ** -24
@@ -69,94 +63,14 @@ DIMS = (4, 8, 16, 32, 64, 128)
 SORT_FROM_ROWS = 4096          # uniq.cu kSortFromRows
 SEGMENTED_ABOVE = 1 << 24      # kmeans.cu / ops.kmeans_accumulate: segmented form when K * N > 2^24
 
-TEMPLATED = ("kmeans_accumulate_kernel", "kmeans_segsum_kernel", "uniq_kernel", "uniq_sorted_kernel")
-PLAIN = ("kmeans_keys_kernel", "kmeans_finalize_kernel", "uniq_keys_kernel")
+FAMILIES = ("kmeans_accumulate_kernel", "kmeans_segsum_kernel", "uniq_kernel", "uniq_sorted_kernel",   # templates
+            "kmeans_keys_kernel", "kmeans_finalize_kernel", "uniq_keys_kernel")                       # plain kernels
 KM_FAMILY = ("kmeans_accumulate_kernel", "kmeans_segsum_kernel", "kmeans_keys_kernel")
 UQ_FAMILY = ("uniq_kernel", "uniq_sorted_kernel", "uniq_keys_kernel")
 
 
-@pytest.fixture(scope="module")
-def lib_mod():
-    import __graft_entry__ as g
-    if not os.path.isfile(LIB):
-        g.build()
-    from hidvae_b200 import _lib
-    return _lib
-
-
-@pytest.fixture(scope="module")
-def ops(lib_mod):
-    from hidvae_b200 import ops as _ops
-    return _ops
-
-
 def _stream():
     return torch.cuda.current_stream().cuda_stream
-
-
-# ---------------------------------------------------------------------------------------------------------------------
-# kernel names: torch.profiler (demangled) and cuobjdump (mangled)
-# ---------------------------------------------------------------------------------------------------------------------
-_DEMANGLED = re.compile(r"\b(" + "|".join(TEMPLATED) + r")<([^<>]*)>")
-_DEMANGLED_PLAIN = re.compile(r"\b(" + "|".join(PLAIN) + r")\(")
-_MANGLED = re.compile(r"\d(" + "|".join(TEMPLATED) + r")I((?:L[ib]-?\d+E)+)E")
-_MANGLED_PLAIN = re.compile(r"\d(" + "|".join(PLAIN) + r")E")
-
-
-def _norm_arg(a):
-    a = a.strip().replace(" ", "")
-    m = re.fullmatch(r"\((bool|int)\)(-?\d+)", a)
-    if m:
-        return ("true" if m.group(2) != "0" else "false") if m.group(1) == "bool" else m.group(2)
-    return a
-
-
-def normalise(name):
-    m = _DEMANGLED.search(name)
-    if m is not None:
-        return f"{m.group(1)}<{','.join(_norm_arg(a) for a in m.group(2).split(','))}>"
-    m = _DEMANGLED_PLAIN.search(name)
-    return None if m is None else m.group(1)
-
-
-def shipped_kernels(symbols_text):
-    out = set()
-    for fam, args in _MANGLED.findall(symbols_text):
-        vals = [("true" if v != "0" else "false") if t == "b" else v for t, v in re.findall(r"L([ib])(-?\d+)E", args)]
-        out.add(f"{fam}<{','.join(vals)}>")
-    out |= set(_MANGLED_PLAIN.findall(symbols_text))
-    return out
-
-
-class Launches(NamedTuple):
-    names: set
-    recorded: bool
-
-
-def profiled(fn):
-    """Run fn() once under torch.profiler (CPU + CUDA activity); returns (fn's result, Launches)."""
-    from torch.profiler import ProfilerActivity, profile
-    torch.cuda.synchronize()
-    with profile(activities=[ProfilerActivity.CPU, ProfilerActivity.CUDA]) as prof:
-        result = fn()
-        torch.cuda.synchronize()
-    names, recorded = set(), False
-    for ev in prof.events():
-        if ev.device_type == torch.autograd.DeviceType.CUDA:
-            recorded = True
-        n = normalise(ev.name)
-        if n is not None:
-            names.add(n)
-    return result, Launches(names, recorded)
-
-
-def assert_launched(launches, expected, family):
-    """`expected` ran, and no other kernel of `family`.  Returns the skip reason when the profiler saw no CUDA kernel."""
-    if not launches.recorded:
-        return "torch.profiler recorded no CUDA kernel on this machine: kernel-name assertion not possible (numbers checked)"
-    seen = {n for n in launches.names if n.split("<")[0] in family}
-    assert seen == set(expected), f"expected exactly {sorted(expected)} of {family}, launched {sorted(seen)}"
-    return None
 
 
 def report(tag, ratios):
@@ -698,15 +612,18 @@ def test_uniqueness_as_wired(ops, b):
     feats = torch.randn(b, 32, generator=g).cuda().requires_grad_(True)
     wired = ids.cuda().transpose(0, 1)
     assert not wired.is_contiguous()
-    loss, launches = profiled(lambda: ops.uniqueness_loss(wired, feats, 0.1, 1.5))
-    grad, launches_b = profiled(lambda: torch.autograd.grad(loss, feats)[0])
+
+    def forward_backward():
+        loss = ops.uniqueness_loss(wired, feats, 0.1, 1.5)
+        return loss, torch.autograd.grad(loss, feats)[0]
+
+    (loss, grad), launches = profiled(forward_backward)
     ref = uniq_reference(wired, feats, 0.1, 1.5)
     assert ref.pairs == 1
     stats = ops.uniq_stats(wired, feats.detach(), 0.1)
     check_uniq(f"as-wired-B{b}", ref, stats, loss, grad, feats.detach(), 32, 0.1, 1.5)
     assert float(ops.count_rows_with_later_twin(wired)) == 1.0
-    skip = assert_launched(Launches(launches.names | launches_b.names, launches.recorded), {"uniq_kernel<false>", "uniq_kernel<true>"},
-                           UQ_FAMILY)
+    skip = assert_launched(launches, {"uniq_kernel<false>", "uniq_kernel<true>"}, UQ_FAMILY)
     if skip:
         pytest.skip(skip)
 
@@ -941,14 +858,8 @@ def test_argument_checks(ops):
 def test_every_kmeans_uniq_kernel_has_a_cell():
     """Every k-means and uniqueness kernel in the built library (16 instantiations of the four templates, three plain
     kernels) is the expected kernel of some cell of this file (CPU only: reads the library with cuobjdump)."""
-    tool = shutil.which("cuobjdump") or os.path.join(os.environ.get("CUDA_HOME", "/usr/local/cuda"), "bin", "cuobjdump")
-    if not os.path.isfile(LIB):
-        pytest.skip(f"{os.path.relpath(LIB, ROOT)} is not built")
-    if not os.path.isfile(tool):
-        pytest.skip("cuobjdump not found")
-    text = subprocess.run([tool, "-symbols", LIB], check=True, capture_output=True, text=True).stdout
-    shipped = shipped_kernels(text)
-    assert {s.split("<")[0] for s in shipped} == set(TEMPLATED + PLAIN), sorted(shipped)
+    shipped = {k for k in shipped_kernels() if family(k) in FAMILIES}
+    assert {family(s) for s in shipped} == set(FAMILIES), sorted(shipped)
     assert len(shipped) == 16 + 3, sorted(shipped)
     covered = {"kmeans_finalize_kernel"} if FINALIZE else set()
     for form, d, _ in KM_CELLS:
@@ -958,18 +869,3 @@ def test_every_kmeans_uniq_kernel_has_a_cell():
     unreached = sorted(shipped - covered)
     assert not unreached, f"{len(unreached)} of {len(shipped)} shipped kernels have no test cell: {unreached}"
     assert not sorted(covered - shipped), f"cells expect kernels the library does not ship: {sorted(covered - shipped)}"
-
-
-def test_kernel_name_normalisation():
-    assert normalise("void hv::(anonymous namespace)::kmeans_segsum_kernel<(int)64>(float const*, long, unsigned long "
-                     "const*, unsigned int const*, int, float*, float*)") == "kmeans_segsum_kernel<64>"
-    assert normalise("void hv::(anonymous namespace)::uniq_kernel<false>(hv::(anonymous namespace)::UniqArgs, double*)") == \
-        "uniq_kernel<false>"
-    assert normalise("void hv::(anonymous namespace)::uniq_sorted_kernel<(bool)1>(hv::UniqArgs)") == "uniq_sorted_kernel<true>"
-    assert normalise("hv::(anonymous namespace)::uniq_keys_kernel(hv::(anonymous namespace)::UniqArgs, unsigned long*, "
-                     "unsigned int*)") == "uniq_keys_kernel"
-    assert normalise("void cub::DeviceRadixSortOnesweepKernel<int>(int)") is None
-    assert shipped_kernels("_ZN2hv41_GLOBAL__N__b0c6ceb8_9_kmeans_cu_900813ab20kmeans_segsum_kernelILi64EEEvPKflPKmPKjiPfS8_ "
-                           "_ZN2hv39_GLOBAL__N__bdcb109d_7_uniq_cu_e4a9325011uniq_kernelILb0EEEvNS0_8UniqArgsEPdPKdfPKfPf "
-                           "_ZN2hv39_GLOBAL__N__bdcb109d_7_uniq_cu_e4a9325016uniq_keys_kernelENS0_8UniqArgsEPmPj") == \
-        {"kmeans_segsum_kernel<64>", "uniq_kernel<false>", "uniq_keys_kernel"}

@@ -10,7 +10,7 @@ import numpy as np
 import pytest
 import torch
 
-from helpers import check_ids, make_codebooks, npz, oracle_levels, t, unit_rows
+from helpers import check_ids, make_codebooks, npz, oracle_levels, ops, t, unit_rows
 from oracle import rq as O
 
 pytestmark = pytest.mark.gpu
@@ -19,12 +19,6 @@ MODES = {"ste": O.MODE_STE, "rot": O.MODE_ROTATION_TRICK}
 ALGOS = ["simt", "tcgen05"]
 VAL = dict(rtol=1e-5, atol=1e-6)
 GCB = dict(rtol=1e-4, atol=1e-5)
-
-
-@pytest.fixture(scope="module")
-def ops():
-    from hidvae_b200 import ops as _ops
-    return _ops
 
 
 def _dev(x):

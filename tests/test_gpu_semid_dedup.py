@@ -14,23 +14,9 @@ import os
 import pytest
 import torch
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+from helpers import ROOT, lib_mod, ops, profiled
+
 gpu = pytest.mark.gpu
-
-
-@pytest.fixture(scope="module")
-def lib_mod():
-    import __graft_entry__ as g
-    if not os.path.isfile(os.path.join(ROOT, "hid-vae_b200", "libhidvae_b200.so")):
-        g.build()
-    from hidvae_b200 import _lib
-    return _lib
-
-
-@pytest.fixture(scope="module")
-def ops(lib_mod):
-    from hidvae_b200 import ops as _ops
-    return _ops
 
 
 # ---------------------------------------------------------------------------------------------------------------------
@@ -319,17 +305,12 @@ def test_deterministic_and_graph_capturable(ops, bench_table):
 
 @gpu
 def test_profiler_sees_only_dedup_and_cub_kernels(ops):
-    from torch.profiler import ProfilerActivity, profile
     ids = make_ids("few", 1 << 20, 3, 8, seed=5)
     ops.semid_dedup(ids, 8)
-    torch.cuda.synchronize()
-    with profile(activities=[ProfilerActivity.CUDA]) as prof:
-        ops.semid_dedup(ids, 8)
-        torch.cuda.synchronize()
-    kernels = {ev.name for ev in prof.events() if ev.device_type == torch.autograd.DeviceType.CUDA
-               and not ev.name.lower().startswith(("memset", "memcpy"))}
-    if not kernels:
+    _, launches = profiled(lambda: ops.semid_dedup(ids, 8))
+    if not launches.recorded:
         pytest.skip("torch.profiler recorded no CUDA kernel on this machine")
+    kernels = launches.kernels
     ours = {k for k in kernels if "dedup_" in k}
     assert {k for k in kernels if k not in ours and "cub::" not in k} == set(), sorted(kernels)
     for name in ("dedup_keys_kernel", "dedup_flags_kernel", "dedup_runs_kernel", "dedup_finish_kernel"):

@@ -21,10 +21,6 @@ B32 = 2^-7 * max_c (sum_j |W3[c, j]| |u_j| + |b3[c]|) (the fp16 rounding of ever
 eight stored layers); every disagreement must be a row whose fp32 top-2 gap is below 2 B32, and at least 99 % of the
 predictions of each level agree.
 """
-import os
-import re
-import shutil
-import subprocess
 import types
 
 import pytest
@@ -32,11 +28,12 @@ import torch
 import torch.nn.functional as F
 from torch import nn
 
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-LIB = os.path.join(ROOT, "hid-vae_b200", "libhidvae_b200.so")
+from helpers import profiled, shipped_kernels
+
 D, FIRST_HIDDEN, COUNTS = 32, 512, (38, 168, 348)
 N_FP64 = 148 * 128 + 77                     # crosses the 18,944-row sub-chunk boundary, ragged last tile
 CHUNK_ROWS = 148 * 128
+FAMILIES = ("tag_gate_kernel", "tag_gemm_kernel", "tag_pack_kernel")
 KERNELS = {f"tag_gemm_kernel<{k}>" for k in range(5)} | {"tag_gate_kernel", "tag_pack_kernel"}
 # which kernels a forward launches, by use_norm
 LAUNCHED = {True: {"tag_gate_kernel", "tag_gemm_kernel<0>", "tag_gemm_kernel<1>", "tag_gemm_kernel<2>", "tag_gemm_kernel<4>"},
@@ -124,19 +121,6 @@ def top2_gap(logits):
     return t[:, 0] - t[:, 1]
 
 
-def kernels_of(fn):
-    from torch.profiler import ProfilerActivity, profile
-    with profile(activities=[ProfilerActivity.CUDA]) as prof:
-        fn()
-        torch.cuda.synchronize()
-    names = set()
-    for e in prof.events():
-        m = re.search(r"\b(tag_[a-z_]+_kernel)(?:<(?:\(int\))?(\d+)>)?", e.name)
-        if m:
-            names.add(m.group(1) + (f"<{m.group(2)}>" if m.group(2) else ""))
-    return names
-
-
 def _fused(model, emb, logits=True):
     from hidvae_b200 import ops
     with torch.no_grad():
@@ -163,7 +147,7 @@ def test_against_fp64(norm, regime):
     model.tag_inference_precision = "fused"
     _regime(model, regime)
     emb = _emb(N_FP64)
-    launched = kernels_of(lambda: _fused(model, emb))
+    launched = profiled(lambda: _fused(model, emb))[1].names
     assert LAUNCHED[norm] <= launched, launched
     pred, conf, logits = _fused(model, emb)
     near_ties = 0
@@ -349,25 +333,12 @@ def test_kernel_cell(kernel):
     model.tag_inference_precision = "fused"
     emb = _emb(300, seed=3)
     model._tag_image = None
-    names = kernels_of(lambda: _fused(model, emb, logits=False))   # packs (tag_pack_kernel) and runs
+    names = profiled(lambda: _fused(model, emb, logits=False))[1].names   # packs (tag_pack_kernel) and runs
     assert kernel in names, names
 
 
-def shipped_tag_kernels(symbols_text):
-    out = set()
-    for name, arg in re.findall(r"\d(tag_[a-z_]+_kernel)(?:ILi(-?\d+)EE)?", symbols_text):
-        out.add(name + (f"<{arg}>" if arg else ""))
-    return out
-
-
 def test_every_shipped_tag_kernel_has_a_cell():
-    tool = shutil.which("cuobjdump") or os.path.join(os.environ.get("CUDA_HOME", "/usr/local/cuda"), "bin", "cuobjdump")
-    if not os.path.isfile(LIB):
-        pytest.skip("libhidvae_b200.so is not built")
-    if not os.path.isfile(tool):
-        pytest.skip("cuobjdump not found")
-    text = subprocess.run([tool, "-symbols", LIB], check=True, capture_output=True, text=True).stdout
-    assert shipped_tag_kernels(text) == KERNELS
+    assert {k for k in shipped_kernels() if k.startswith("tag_")} == KERNELS
 
 
 # ---------------------------------------------------------------------------------------------------------------------
